@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — LM iterations/s and residual+Jacobian Gobs/s of the calibration solve.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A "step" is ONE Levenberg-Marquardt iteration (Schur elimination, reduced solve,
 back-substitution, residual+Jacobian+normal-equation pass at the candidate point,
@@ -33,6 +33,11 @@ The JSON line also carries:
 
 `--impl reference` times the CPU restatement of the reference's Ceres path (the
 reference itself cannot be built: Ceres/Eigen/OpenCV are absent) on the host cores.
+
+`--dump-outputs DIR` writes the parameters the timed LM iterations end at, as a caller of the
+solve receives them, to DIR/intrinsics.npy (C x 9), DIR/cam_rt.npy (C x 6) and DIR/board_rt.npy
+(F x 6), float64.  The workload is synthesised from fixed seeds, so two builds run with the same
+arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -46,6 +51,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # the tree may be read-only; the benchmark leaves nothing in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -144,6 +150,13 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def write_outputs(directory, intrinsics, cam_rt, board_rt):
+    """--dump-outputs: the solved parameters as DIR/<name>.npy, float64."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in (("intrinsics", intrinsics), ("cam_rt", cam_rt), ("board_rt", board_rt)):
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def fixed_iteration_options(n, **kw):
     from tscm_calib_b200 import capi
     return capi.default_options(max_num_iterations=int(n), disable_tolerances=1, **kw)
@@ -177,7 +190,10 @@ def run_reference(args):
     sp = synth.config(3, num_frames=frames)
     if args.warmup > 0:
         time_oracle(sp.problem, sp.init_intrinsics, sp.init_cam_rt, sp.init_board_rt, min(args.warmup, 1), threads)
-    dt, _ = time_oracle(sp.problem, sp.init_intrinsics, sp.init_cam_rt, sp.init_board_rt, args.steps, threads)
+    dt, (a, b, c, _) = time_oracle(sp.problem, sp.init_intrinsics, sp.init_cam_rt, sp.init_board_rt, args.steps,
+                                   threads)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, a, b, c)
     gobs = sp.num_observations * args.steps / dt / 1e9
     sample = (f"{frames} of 5000 frames of config 3 ({sp.num_observations} observations), "
               f"{args.steps} LM iterations incl. iteration-0 evaluation, {threads} threads")
@@ -279,6 +295,18 @@ def run_b200(args):
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     launches = solver.launch_count() - launches0
+    if args.dump_outputs:
+        # the point the last timed iteration left on the device; at N > 1 every rank holds the
+        # board poses of its own frames, gathered on rank 0 into the order of the whole problem
+        intr_out, cam_out, board_out = solver.get_parameters()
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, (fr, board_out), group=cpu_group)
+            board_out = np.zeros((sp.problem.num_frames, 6))
+            for frames, part in parts:
+                board_out[frames] = part
+        if rank == 0:
+            write_outputs(args.dump_outputs, intr_out, cam_out, board_out)
     ms_iter = max_over_ranks(ms_iter)
     it_per_s = 1e3 / ms_iter
     value = total_obs * it_per_s / 1e9
@@ -542,7 +570,11 @@ def main():
     ap.add_argument("--stress-frames", type=int, default=20000,
                     help="frames of the config-4 sample timed beside the headline at N = 1 (0 = skip)")
     ap.add_argument("--debug-flags", type=int, default=0, help="tscm_set_debug() flags (4 = no programmatic dependent launch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the parameters the timed iterations end at to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)

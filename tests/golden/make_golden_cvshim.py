@@ -48,5 +48,25 @@ def main():
     print("opencv", cv2.__version__, "pnp costs", np.array(costs).round(8)[:6])
 
 
+def non_orthonormal():
+    """cv_rodrigues_nonortho.npz: cv::Rodrigues of matrices that are not rotations, as the reference
+    hands them over (r3 = r1 x r2 from float-truncated columns, chained pose-graph products)."""
+    rng = np.random.default_rng(5)
+    mats, backs = [], []
+    for k in range(40):
+        v = rng.normal(size=3) * rng.uniform(0.05, 2.5)
+        R, _ = cv2.Rodrigues(v)
+        if k % 2 == 0:
+            M = R.astype(np.float32).astype(np.float64)            # float truncation, Rt_to_R_t style
+            M[:, 2] = np.cross(M[:, 0], M[:, 1])
+        else:
+            M = R + rng.normal(scale=1e-4, size=(3, 3))            # accumulated error of chained products
+        M = np.ascontiguousarray(M)
+        mats.append(M)
+        backs.append(cv2.Rodrigues(M)[0].reshape(3))
+    np.savez_compressed(os.path.join(OUT, "cv_rodrigues_nonortho.npz"), mat=np.stack(mats), back=np.stack(backs))
+
+
 if __name__ == "__main__":
     main()
+    non_orthonormal()

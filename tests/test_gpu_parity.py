@@ -2,10 +2,12 @@
 libtscm_b200.so and is compared with the CPU oracle / the committed golden vectors.
 North-star tolerances: Jacobian 1e-10, per-iteration cost 1e-9 relative, final
 parameters 1e-7 relative, RMS reprojection error 1e-9 px."""
+import os
+
 import numpy as np
 import pytest
 
-from conftest import golden_options, load_golden, rel_err
+from conftest import GOLDEN, golden_options, load_golden, rel_err
 from tscm_calib_b200 import capi, synth
 
 pytestmark = pytest.mark.gpu
@@ -41,7 +43,7 @@ def test_residuals_and_jacobian_match_oracle(oracle, cfg):
 def test_jacobian_matches_mpmath_golden(golden):
     """k_eval_rows against 50-digit central differences and against sympy's symbolic derivative
     of the reference functor (tests/golden/make_golden_sympy.py)."""
-    z = np.load(f"tests/golden/{golden}.npz")
+    z = np.load(os.path.join(GOLDEN, golden + ".npz"))
     for k in range(len(z["r"])):
         p = capi.ProblemArrays(z["board"][k][None, :], [0], [0], z["obs"][k][None, None, :], 1, 1,
                                fixed_camera=-1)

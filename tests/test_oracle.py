@@ -3,11 +3,12 @@ mpmath restatement), against the kernels' host-compiled arithmetic, and against
 domain properties.  Tolerances: per-iteration cost 1e-9 rel, parameters 1e-7 rel,
 Jacobian 1e-10 (BASELINE.json north_star)."""
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
 
-from conftest import golden_options, load_golden, rel_err
+from conftest import GOLDEN, golden_options, load_golden, rel_err
 from tscm_calib_b200 import capi, synth
 from tscm_calib_b200.capi import _dp
 
@@ -60,7 +61,7 @@ def test_jets_and_analytic_jacobian_match_mpmath(oracle, hostmath, golden):
     multi_calib.h:146-195 (make_golden_sympy.py: nothing hand-derived) pin both the Jet autodiff
     and the hand-derived Jacobian, including the theta^2 <= eps Taylor branch of
     AngleAxisRotatePoint."""
-    z = np.load(f"tests/golden/{golden}.npz")
+    z = np.load(os.path.join(GOLDEN, golden + ".npz"))
     n = len(z["r"])
     taylor = 0
     for k in range(n):
