@@ -67,7 +67,8 @@ enum {
   TSCM_ERR_NO_DEVICE = 3,     /* no sm_100 device: there is NO CPU fallback */
   TSCM_ERR_COMM = 4,          /* NCCL failure */
   TSCM_ERR_UNSUPPORTED = 5,
-  TSCM_ERR_NO_CANDIDATE = 6   /* pose graph: no usable candidate (tscm_pose_graph_init) */
+  TSCM_ERR_NO_CANDIDATE = 6,  /* pose graph: no usable candidate (tscm_pose_graph_init) */
+  TSCM_ERR_RANK_DEFICIENT = 7 /* covariance: H is singular (gauge freedom, degenerate board) */
 };
 
 typedef struct tscm_problem {
@@ -199,6 +200,51 @@ int tscm_solver_attach_comm(tscm_solver* solver, int rank, int num_ranks,
 int tscm_solver_p2p_export(tscm_solver* solver, void* handle_64);
 int tscm_solver_p2p_attach(tscm_solver* solver, int rank, int num_ranks, const void* handles);
 int tscm_solver_set_exchange_timeout(tscm_solver* solver, double seconds);
+
+/* ---- parameter covariance ---------------------------------------------------------------
+ * The covariance of the estimate at the current parameters x, as ceres::Covariance reports it:
+ *   Sigma = H^-1,  H = J^T J,
+ * J the Jacobian of all residuals at x with the configured robust loss applied through Ceres'
+ * corrector (the J of the LM step), no LM diagonal.  Only LIVE parameters enter: per camera
+ * [rt(6) unless it is the fixed camera][fx fy cx cy xi lambda alpha] (the layout of
+ * tscm_solver_reduced_system), plus 6 per frame.  Unlike ceres::Covariance on the reference's
+ * 9-wide intrinsic block, b and c are excluded: their Jacobian columns are identically zero
+ * (TS.h:122-125), so that block would be rank deficient.  The fixed camera's rt has no entries.
+ * Returned are the camera block (n x n, n = tscm_solver_reduced_size()) and the 6 x 6 diagonal
+ * block of every board pose; camera x board and board x board cross blocks are not computed.
+ * It is evaluated as Sigma = D (D H D)^-1 D with the Jacobi scales D of the LM solve:
+ *   camera block  D_c S~^-1 D_c,   S~ the undamped scaled reduced camera system,
+ *   board f       D_e,f (V~_f^-1 + Y~_f S~^-1 Y~_f^T) D_e,f,   Y~_f = V~_f^-1 W~_f.
+ * Sigma is raw, as in Ceres; standard deviations in OpenCV's sense (calibrateCameraExtended) are
+ * sqrt(residual_variance * diag(Sigma)) with
+ *   residual_variance = sum |r|^2 / (2N - (n + 6F)),
+ * r the plain (loss-free) residuals, N observations and F frames over all shards and ranks (NaN
+ * when 2N <= n + 6F).
+ * TSCM_ERR_RANK_DEFICIENT (nothing written): a pivot of the LDL^T of S~ or of some V~_f is
+ * <= 1e-14 x the largest diagonal entry of that matrix (the default
+ * min_reciprocal_condition_number of ceres::Covariance) — e.g. fixed_camera = -1 leaves a
+ * 6-dimensional gauge freedom, or a board pose is not determined by its views.
+ * Host pointers.  The solver's state is unaffected: a later tscm_solver_run() behaves as if this
+ * call had not been made. */
+typedef struct tscm_covariance {
+  double* camera;            /* optional, n x n row-major, n = tscm_solver_reduced_size(), live order */
+  double* board;             /* optional, F x 6 x 6 row-major: covariance of board_rt[f] */
+  double residual_variance;  /* out: sum |r|^2 / (2N - n_free), plain residuals */
+  double kernel_ms;          /* out: device time of the covariance kernels (CUDA events) */
+} tscm_covariance;
+
+/* At the parameters on the device (after tscm_solver_run(): the solution).  On a num_gpus group
+ * `board` holds all F frames in problem order.  Multi-process ranks: collective like run(); the
+ * camera block is identical on every rank, `board` holds the rank's own frames, indexed as in
+ * tscm_solver_get_parameters(). */
+int tscm_solver_covariance(tscm_solver* solver, tscm_covariance* cov);
+/* One-shot form at the given parameters (host pointers, not modified), through the solver cache
+ * of tscm_solve(): after a tscm_solve() of the same structure it only uploads observations and
+ * parameters — no new solver, no graph capture.  (Named apart from the struct: in C a function
+ * and a typedef cannot share the name tscm_covariance.) */
+int tscm_compute_covariance(const tscm_problem* problem, const tscm_options* options, const double* intrinsics,
+                            const double* cam_rt, const double* board_rt, tscm_covariance* cov,
+                            int device);
 
 /* ---- inspection entry points (used by the parity tests and the bench) ---- */
 

@@ -77,6 +77,16 @@ class TscmSummary(C.Structure):
     ]
 
 
+class TscmCovariance(C.Structure):
+    """tscm_covariance (include/tscm.h)."""
+    _fields_ = [
+        ("camera", c_double_p),
+        ("board", c_double_p),
+        ("residual_variance", C.c_double),
+        ("kernel_ms", C.c_double),
+    ]
+
+
 class TscmRemapJob(C.Structure):
     """tscm_remap_job (include/tscm.h): one block of a remap table."""
     _fields_ = [
@@ -316,6 +326,11 @@ def load_library(path: str | None = None):
     lib.tscm_solver_reduced_system.restype = C.c_int
     lib.tscm_solver_reprojection_error.argtypes = [C.c_void_p, c_double_p, c_double_p, c_double_p]
     lib.tscm_solver_reprojection_error.restype = C.c_int
+    lib.tscm_solver_covariance.argtypes = [C.c_void_p, P(TscmCovariance)]
+    lib.tscm_solver_covariance.restype = C.c_int
+    lib.tscm_compute_covariance.argtypes = [P(TscmProblem), P(TscmOptions), c_double_p, c_double_p,
+                                            c_double_p, P(TscmCovariance), C.c_int]
+    lib.tscm_compute_covariance.restype = C.c_int
     lib.tscm_solver_time_stage.argtypes = [C.c_void_p, C.c_int, C.c_int, c_double_p]
     lib.tscm_solver_time_stage.restype = C.c_int
     lib.tscm_solver_launch_count.argtypes = [C.c_void_p]
@@ -349,20 +364,65 @@ EXPORTED_SYMBOLS = [
     "tscm_last_error", "tscm_version", "tscm_cache_configure", "tscm_cache_release",
     "tscm_host_alloc", "tscm_host_free", "tscm_solver_set_exchange_timeout",
     "tscm_solver_set_schur_form", "tscm_set_debug", "tscm_pose_graph_init", "tscm_mono_init",
+    "tscm_solver_covariance", "tscm_compute_covariance",
 ]
+
+ERR_RANK_DEFICIENT = 7   # TSCM_ERR_RANK_DEFICIENT
 
 SCHUR_FORM = {"auto": 0, "rows": 1, "fused": 2, "pairs": 3}
 
 
 class TscmError(RuntimeError):
-    pass
+    def __init__(self, message: str, code: int = 0):
+        super().__init__(message)
+        self.code = code
 
 
 def check(rc: int, lib=None):
     if rc != 0:
         lib = lib or load_library()
         msg = lib.tscm_last_error()
-        raise TscmError(f"tscm error {rc}: {msg.decode() if msg else ''}")
+        raise TscmError(f"tscm error {rc}: {msg.decode() if msg else ''}", rc)
+
+
+@dataclass
+class CovarianceResult:
+    """Output of tscm_solver_covariance / tscm_compute_covariance (include/tscm.h)."""
+    camera: np.ndarray             # n x n, live order (tscm_solver_reduced_size)
+    board: np.ndarray | None       # F x 6 x 6
+    residual_variance: float       # sum |r|^2 / (2N - n_free), plain residuals
+    kernel_ms: float
+
+
+def _covariance_buffers(n: int, F: int, boards: bool):
+    cam = np.zeros((n, n))
+    brd = np.zeros((F, 6, 6)) if boards else None
+    c = TscmCovariance(_dp(cam), _dp(brd) if boards else None, 0.0, 0.0)
+    return cam, brd, c
+
+
+def live_columns(problem: "ProblemArrays"):
+    """(camera, index in [rt 6 | intrinsics 9]) of every live column of the reduced system."""
+    cols = []
+    for m in range(problem.num_cameras):
+        ks = range(6, 13) if m == problem.fixed_camera else range(13)
+        cols += [(m, k) for k in ks]
+    return cols
+
+
+def camera_std_dev(problem: "ProblemArrays", cov, residual_variance: float | None = None) -> np.ndarray:
+    """C x 15 standard deviations [rt 6 | fx fy cx cy xi lambda alpha b c] in OpenCV's sense,
+    sqrt(residual_variance * diag(Sigma)), from the live camera block (a CovarianceResult or the
+    n x n matrix).  Entries that are not free (the fixed camera's rt, b, c) are 0."""
+    if isinstance(cov, CovarianceResult):
+        if residual_variance is None:
+            residual_variance = cov.residual_variance
+        cov = cov.camera
+    out = np.zeros((problem.num_cameras, 15))
+    d = np.diag(np.asarray(cov))
+    for i, (m, k) in enumerate(live_columns(problem)):
+        out[m, k] = np.sqrt(residual_variance * d[i])
+    return out
 
 
 class Solver:
@@ -469,6 +529,13 @@ class Solver:
         check(self.lib.tscm_solver_reprojection_error(self.h, _dp(per), C.byref(overall),
                                                       C.byref(rms)), self.lib)
         return per, overall.value, rms.value
+
+    def covariance(self, boards: bool = True) -> CovarianceResult:
+        """tscm_solver_covariance(): covariance of the live parameters at the current point.
+        Raises TscmError with code ERR_RANK_DEFICIENT when J^T J is singular."""
+        cam, brd, c = _covariance_buffers(self.reduced_size(), self.problem.num_frames, boards)
+        check(self.lib.tscm_solver_covariance(self.h, C.byref(c)), self.lib)
+        return CovarianceResult(cam, brd, c.residual_variance, c.kernel_ms)
 
     def time_stage(self, stage: int, repeats: int) -> float:
         ms = C.c_double()
@@ -609,6 +676,22 @@ def solve(problem: ProblemArrays, intrinsics, cam_rt, board_rt, options: TscmOpt
     check(lib.tscm_solve(C.byref(problem.c), C.byref(options), _dp(a), _dp(b), _dp(c),
                          C.byref(buf.c), device), lib)
     return a, b, c, buf.result()
+
+
+def covariance(problem: ProblemArrays, intrinsics, cam_rt, board_rt, options: TscmOptions | None = None,
+               device: int = -1, boards: bool = True) -> CovarianceResult:
+    """One-shot tscm_compute_covariance() at the given parameters, through the solver cache of
+    solve(): after a solve() of the same structure only the data are uploaded."""
+    lib = load_library()
+    options = options or default_options()
+    a = np.ascontiguousarray(intrinsics, dtype=np.float64).reshape(problem.num_cameras, 9)
+    b = np.ascontiguousarray(cam_rt, dtype=np.float64).reshape(problem.num_cameras, 6)
+    c = np.ascontiguousarray(board_rt, dtype=np.float64).reshape(problem.num_frames, 6)
+    n = sum(7 if m == problem.fixed_camera else 13 for m in range(problem.num_cameras))
+    cam, brd, cv = _covariance_buffers(n, problem.num_frames, boards)
+    check(lib.tscm_compute_covariance(C.byref(problem.c), C.byref(options), _dp(a), _dp(b), _dp(c),
+                                      C.byref(cv), device), lib)
+    return CovarianceResult(cam, brd, cv.residual_variance, cv.kernel_ms)
 
 
 def solve_resident(problem: ProblemArrays, intrinsics, cam_rt, board_rt, options: TscmOptions | None = None,

@@ -38,6 +38,7 @@
 #include "tscm_pair_lists.h"
 #include "tscm_remap.cuh"
 #include "tscm_posegraph.cuh"
+#include "tscm_covariance.cuh"
 #include "tscm_internal.h"
 
 namespace {
@@ -272,6 +273,13 @@ struct tscm_solver {
   std::vector<int> kid_frame;       // [n + 1] frame range of every shard
   std::vector<std::vector<ObsSegment>> kid_seg;
   bool is_kid = false;
+  // covariance (tscm_solver_covariance), allocated on first use
+  double* d_cov_fac = nullptr;      // [NL][NL] LDL^T factor of S~, mirrored
+  double* d_cov_sinv = nullptr;     // [NL][NL] S~^-1 (scaled)
+  double* d_cov_cam = nullptr;      // [NL][NL] camera block, unscaled
+  double* d_cov_board = nullptr;    // [F][36] board blocks, unscaled
+  int* d_cov_flag = nullptr;
+  cudaEvent_t cov_ev[2] = {nullptr, nullptr};
 };
 
 namespace {
@@ -563,6 +571,26 @@ int run_initial(tscm_solver* s) {
   return TSCM_OK;
 }
 
+// Evaluate the point in set `cur` with the configured loss, compute the Jacobi scaling there (as
+// iteration 0 does) and assemble the reduced camera system at `radius` into d_Sr (radius = +inf:
+// the undamped system).  Asynchronous; on a sharded solve every shard must make the same call.
+int assemble_at(tscm_solver* s, double radius) {
+  const int cur = s->x_in_set1 ? 1 : 0;
+  LmState* tmp = s->h_state + 1;
+  std::memset(tmp, 0, sizeof(LmState));
+  tmp->cur = cur;
+  CUDA_TRY(cudaMemcpyAsync(s->d_state, tmp, sizeof(LmState), cudaMemcpyHostToDevice, s->stream));
+  launch_evaluation(s, 2 + cur, 1);
+  RC_TRY(launch_eval_allreduce(s, 2 + cur));
+  const int n = s->P.F * 6 + s->P.C * 13;
+  k_jacobi_scale<<<(n + 255) / 256, 256, 0, s->stream>>>(s->P, s->ps[0], s->ps[1], s->d_state, s->lm,
+                                                        s->d_scale_e, s->d_scale_c);
+  s->launches += 1;
+  launch_schur(s, radius);
+  RC_TRY(launch_schur_allreduce(s, radius));
+  return TSCM_OK;
+}
+
 int fetch_state(tscm_solver* s) {
   CUDA_TRY(cudaMemcpyAsync(s->h_state, s->d_state, sizeof(LmState), cudaMemcpyDeviceToHost, s->stream));
   CUDA_TRY(cudaStreamSynchronize(s->stream));
@@ -745,8 +773,10 @@ void free_shard(tscm_solver* s) {
   if (s->comm && nccl().ok) nccl().CommDestroy(s->comm);
   for (int r = 0; r < kP2PMaxRanks; ++r)
     if (s->p2p_ipc[r]) cudaIpcCloseMemHandle(s->p2p_ipc[r]);
-  for (int k = 0; k < 2; ++k)
+  for (int k = 0; k < 2; ++k) {
     if (s->poll_ev[k]) cudaEventDestroy(s->poll_ev[k]);
+    if (s->cov_ev[k]) cudaEventDestroy(s->cov_ev[k]);
+  }
   if (s->arena.base) cudaFree(s->arena.base);
   for (void* p : s->extra) cudaFree(p);
   if (s->d_mailbox) cudaFree(s->d_mailbox);
@@ -1195,6 +1225,72 @@ int upload_all_observations(tscm_solver* s, const double* obs_xy) {
   });
 }
 
+// The cached solver of this structure, taken out of the cache (nobody else may use it meanwhile),
+// or nullptr.
+tscm_solver* cache_checkout(const tscm_problem* p, int device, int ngpu) {
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  for (size_t i = 0; i < g_cache.size(); ++i) {
+    CacheEntry& e = g_cache[i];
+    if (e.device == device && e.num_gpus == ngpu && same_structure(e.solver, p)) {
+      tscm_solver* s = e.solver;
+      g_cache.erase(g_cache.begin() + i);
+      return s;
+    }
+  }
+  return nullptr;
+}
+// Back into the cache (keep = the solver is in a usable state), or destroyed.
+void cache_checkin(tscm_solver* s, int device, int ngpu, bool keep) {
+  std::lock_guard<std::mutex> lock(g_cache_mu);
+  if (keep && g_cache_max > 0) {
+    while ((int)g_cache.size() >= g_cache_max) cache_evict_oldest_locked();
+    CacheEntry e;
+    e.solver = s; e.device = device; e.num_gpus = ngpu; e.stamp = ++g_cache_clock;
+    g_cache.push_back(e);
+  } else {
+    destroy_solver(s);
+  }
+}
+
+// ---------------------------------------------------------------------------
+// covariance (tscm_covariance.cuh)
+// ---------------------------------------------------------------------------
+int ensure_cov_buffers(tscm_solver* k) {
+  if (k->d_cov_fac) return TSCM_OK;
+  const size_t NL = (size_t)k->P.NL;
+  if (k->P.NL > kCovMaxNL) { set_error("covariance: %d live parameters exceed %d", k->P.NL, kCovMaxNL); return TSCM_ERR_UNSUPPORTED; }
+  if (cov_factor_smem(k->P.NL) > k->smem_optin) { set_error("covariance needs %zu bytes of shared memory", cov_factor_smem(k->P.NL)); return TSCM_ERR_UNSUPPORTED; }
+  Arena a;
+  a.want(&k->d_cov_fac, NL * NL);
+  a.want(&k->d_cov_sinv, NL * NL);
+  a.want(&k->d_cov_cam, NL * NL);
+  a.want(&k->d_cov_board, (size_t)k->F * 36);
+  a.want(&k->d_cov_flag, 1);
+  RC_TRY(a.commit(k->stream));
+  k->extra.push_back(a.base);
+  RC_TRY(set_smem_attr((const void*)k_cov_factor, cov_factor_smem(k->P.NL)));
+  for (int e = 0; e < 2; ++e) CUDA_TRY(cudaEventCreate(&k->cov_ev[e]));
+  return TSCM_OK;
+}
+
+// The three covariance kernels on the system assemble_at(+inf) left in d_Sr.  Asynchronous.
+int launch_covariance(tscm_solver* k) {
+  const int NL = k->P.NL, cur = k->x_in_set1 ? 1 : 0;
+  CUDA_TRY(cudaMemsetAsync(k->d_cov_flag, 0, sizeof(int), k->stream));
+  CUDA_TRY(cudaEventRecord(k->cov_ev[0], k->stream));
+  k_cov_factor<<<1, kCovFactorThreads, cov_factor_smem(NL), k->stream>>>(NL, k->solve.nbk, k->d_Sr, k->d_cov_fac,
+                                                                          k->d_cov_flag);
+  k_cov_inverse<<<(NL + kCovInvWarps - 1) / kCovInvWarps, 32 * kCovInvWarps, 0, k->stream>>>(
+      k->P, k->d_scale_c, k->d_cov_fac, k->d_cov_flag, k->d_cov_sinv, k->d_cov_cam);
+  k_cov_frames<<<(k->F + kCovFrameWarps - 1) / kCovFrameWarps, 32 * kCovFrameWarps, 0, k->stream>>>(
+      k->P, k->ps[cur], k->d_scale_e, k->d_scale_c, k->schur.frame_rec, k->schur.Fpad, k->d_cov_sinv, k->d_cov_flag,
+      k->d_cov_board);
+  CUDA_TRY(cudaEventRecord(k->cov_ev[1], k->stream));
+  k->launches += 3;
+  CUDA_TRY(cudaGetLastError());
+  return TSCM_OK;
+}
+
 }  // namespace
 
 // ---- helpers shared with the other translation units (tscm_internal.h) ----
@@ -1510,20 +1606,8 @@ int tscm_solve(const tscm_problem* problem, const tscm_options* options, double*
   if (device < 0) CUDA_TRY(cudaGetDevice(&device));
   const int ngpu = std::max(1, options->num_gpus);
   // ---- solver: cached for this structure, or new ---------------------------------------------
-  tscm_solver* s = nullptr;
-  bool hit = false;
-  {
-    std::lock_guard<std::mutex> lock(g_cache_mu);
-    for (size_t i = 0; i < g_cache.size(); ++i) {
-      CacheEntry& e = g_cache[i];
-      if (e.device == device && e.num_gpus == ngpu && same_structure(e.solver, problem)) {
-        s = e.solver;
-        g_cache.erase(g_cache.begin() + i);     // checked out: nobody else may use it meanwhile
-        hit = true;
-        break;
-      }
-    }
-  }
+  tscm_solver* s = cache_checkout(problem, device, ngpu);
+  const bool hit = s != nullptr;
   const double ms_lookup = ms_since(t0);
   int rc = TSCM_OK;
   if (hit) {
@@ -1542,17 +1626,7 @@ int tscm_solve(const tscm_problem* problem, const tscm_options* options, double*
   const double ms_run = ms_since(t0);
   if (!rc) rc = tscm_solver_get_parameters(s, intrinsics, cam_rt, board_rt);
   const double ms_get = ms_since(t0);
-  if (s) {
-    std::lock_guard<std::mutex> lock(g_cache_mu);
-    if (rc == TSCM_OK && g_cache_max > 0) {
-      while ((int)g_cache.size() >= g_cache_max) cache_evict_oldest_locked();
-      CacheEntry e;
-      e.solver = s; e.device = device; e.num_gpus = ngpu; e.stamp = ++g_cache_clock;
-      g_cache.push_back(e);
-    } else {
-      destroy_solver(s);
-    }
-  }
+  if (s) cache_checkin(s, device, ngpu, rc == TSCM_OK);
   if (g_debug & 1)
     std::fprintf(stderr, "[tscm_solve] %s: lookup %.2f  create/upload %.2f  set %.2f  run %.2f  get %.2f  total %.2f ms\n",
                  hit ? "cached solver" : "new solver", ms_lookup, ms_create - ms_lookup, ms_set - ms_create,
@@ -1704,20 +1778,7 @@ int tscm_solver_reduced_system(tscm_solver* s, double radius, double* lhs, doubl
   if (!s || !(radius > 0.0)) { set_error("bad arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_reduced_system");
   CUDA_TRY(cudaSetDevice(s->device));
-  // Evaluate the point in set `cur`, compute Jacobi scaling there (as iteration 0 does).
-  const int cur = s->x_in_set1 ? 1 : 0;
-  LmState* tmp = s->h_state + 1;
-  std::memset(tmp, 0, sizeof(LmState));
-  tmp->cur = cur;
-  CUDA_TRY(cudaMemcpyAsync(s->d_state, tmp, sizeof(LmState), cudaMemcpyHostToDevice, s->stream));
-  launch_evaluation(s, 2 + cur, 1);
-  RC_TRY(launch_eval_allreduce(s, 2 + cur));
-  const int n = s->P.F * 6 + s->P.C * 13;
-  k_jacobi_scale<<<(n + 255) / 256, 256, 0, s->stream>>>(s->P, s->ps[0], s->ps[1], s->d_state, s->lm,
-                                                        s->d_scale_e, s->d_scale_c);
-  s->launches += 1;
-  launch_schur(s, radius);
-  RC_TRY(launch_schur_allreduce(s, radius));
+  RC_TRY(assemble_at(s, radius));
   CUDA_TRY(cudaStreamSynchronize(s->stream));
   CUDA_TRY(cudaGetLastError());
   // the assembled system as k_solve receives it (4x4 tiles of the lower block triangle)
@@ -1787,6 +1848,149 @@ int tscm_solver_reprojection_error(tscm_solver* s, double* per_camera, double* o
   // restore the records of the configured loss for a subsequent run()
   if (L->lm.loss_type || multi_process) RC_TRY(evaluate(false));
   return TSCM_OK;
+}
+
+// Covariance of the live parameters at the current point (DESIGN.md 5e, tscm_covariance.cuh).
+// Collective on a sharded solve, like run(): every shard assembles the undamped system over the
+// usual exchange and inverts S~ redundantly; each shard computes the blocks of its own frames.
+int tscm_solver_covariance(tscm_solver* s, tscm_covariance* out) {
+  DeviceGuard device_guard_;
+  if (!s || !out) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
+  const int C = s->C;
+  tscm_solver* L = lead(s);
+  const int NL = L->P.NL;
+  const bool multi_process = s->kids.empty() && s->num_ranks > 1;
+  // sum |r|^2 of the plain (loss-free) residuals
+  RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
+    CUDA_TRY(cudaSetDevice(k->device));
+    RC_TRY(ensure_cov_buffers(k));
+    const int cur = k->x_in_set1 ? 1 : 0;
+    const LmOptions saved = k->lm;
+    k->lm.loss_type = 0;
+    launch_evaluation(k, 2 + cur, 1);
+    const int rc = launch_eval_allreduce(k, 2 + cur);
+    k->lm = saved;
+    return rc;
+  }));
+  RC_TRY(sync_shards(s));
+  const int cur = L->x_in_set1 ? 1 : 0;
+  CUDA_TRY(cudaSetDevice(L->device));
+  CUDA_TRY(cudaGetLastError());
+  std::vector<double> rec((size_t)C * kCamRec + kCommExtra, 0.0);
+  CUDA_TRY(cudaMemcpy(rec.data(), L->ps[cur].comm, (size_t)C * kCamRec * sizeof(double), cudaMemcpyDeviceToHost));
+  double rr = 0.0;
+  for (int m = 0; m < C; ++m) rr += 2.0 * rec[(size_t)m * kCamRec + kCamCost];
+  // the undamped system under the configured loss (which also restores that loss's records for a
+  // later run()), then the covariance kernels
+  RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
+    CUDA_TRY(cudaSetDevice(k->device));
+    return assemble_at(k, INFINITY);
+  }));
+  RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
+    CUDA_TRY(cudaSetDevice(k->device));
+    return launch_covariance(k);
+  }));
+  RC_TRY(sync_shards(s));
+  int flag = 0;
+  double ms = 0.0;
+  RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
+    CUDA_TRY(cudaSetDevice(k->device));
+    CUDA_TRY(cudaGetLastError());
+    int f = 0;
+    CUDA_TRY(cudaMemcpy(&f, k->d_cov_flag, sizeof(int), cudaMemcpyDeviceToHost));
+    flag |= f;
+    float e = 0.f;
+    CUDA_TRY(cudaEventElapsedTime(&e, k->cov_ev[0], k->cov_ev[1]));
+    ms = std::max(ms, (double)e);
+    return TSCM_OK;
+  }));
+  // global counts: a group knows them; the ranks of a multi-process solve exchange them (and the
+  // frame rank test) through an evaluation record, as tscm_solver_reprojection_error does
+  std::vector<double> count = L->obs_count;
+  double frames = s->F;
+  if (multi_process) {
+    CUDA_TRY(cudaSetDevice(L->device));
+    std::fill(rec.begin(), rec.end(), 0.0);
+    for (int m = 0; m < C; ++m) rec[(size_t)m * kCamRec + kCamErr] = L->obs_count[m];
+    rec[kCamCost] = L->F;
+    rec[(size_t)C * kCamRec] = (flag & 2) ? 1.0 : 0.0;
+    CUDA_TRY(cudaMemcpyAsync(L->ps[cur].comm, rec.data(), rec.size() * sizeof(double), cudaMemcpyHostToDevice, L->stream));
+    RC_TRY(launch_eval_allreduce(L, 2 + cur));
+    CUDA_TRY(cudaStreamSynchronize(L->stream));
+    CUDA_TRY(cudaMemcpy(rec.data(), L->ps[cur].comm, rec.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    for (int m = 0; m < C; ++m) count[m] = rec[(size_t)m * kCamRec + kCamErr];
+    frames = rec[kCamCost];
+    if (rec[(size_t)C * kCamRec] > 0.0) flag |= 2;
+    // restore the records of the configured loss
+    launch_evaluation(L, 2 + cur, 1);
+    RC_TRY(launch_eval_allreduce(L, 2 + cur));
+    CUDA_TRY(cudaStreamSynchronize(L->stream));
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (flag) {
+    set_error((flag & 1) ? "covariance: J^T J is rank deficient in the camera parameters (a gauge freedom: "
+                           "is no camera fixed?)"
+                         : "covariance: J^T J is rank deficient in a board pose (a degenerate board)");
+    return TSCM_ERR_RANK_DEFICIENT;
+  }
+  double N = 0.0;
+  for (int m = 0; m < C; ++m) N += count[m];
+  const double dof = 2.0 * N - (NL + 6.0 * frames);
+  out->residual_variance = dof > 0.0 ? rr / dof : NAN;
+  out->kernel_ms = ms;
+  if (out->camera) {
+    CUDA_TRY(cudaSetDevice(L->device));
+    CUDA_TRY(cudaMemcpy(out->camera, L->d_cov_cam, (size_t)NL * NL * sizeof(double), cudaMemcpyDeviceToHost));
+    for (int r = 0; r < NL; ++r)          // columns are solved independently: average the two triangles
+      for (int c = 0; c < r; ++c) {
+        const double v = 0.5 * (out->camera[(size_t)r * NL + c] + out->camera[(size_t)c * NL + r]);
+        out->camera[(size_t)r * NL + c] = v;
+        out->camera[(size_t)c * NL + r] = v;
+      }
+  }
+  if (out->board) {
+    RC_TRY(for_shards(s, [&](tscm_solver* k, int i) -> int {
+      CUDA_TRY(cudaSetDevice(k->device));
+      double* dst = out->board + (s->kids.empty() ? 0 : (size_t)s->kid_frame[i] * 36);
+      CUDA_TRY(cudaMemcpy(dst, k->d_cov_board, (size_t)k->F * 36 * sizeof(double), cudaMemcpyDeviceToHost));
+      return TSCM_OK;
+    }));
+  }
+  return TSCM_OK;
+}
+
+int tscm_compute_covariance(const tscm_problem* problem, const tscm_options* options, const double* intrinsics,
+                    const double* cam_rt, const double* board_rt, tscm_covariance* cov, int device) {
+  DeviceGuard device_guard_;
+  RC_TRY(validate_problem(problem, true));
+  if (!intrinsics || !cam_rt || !board_rt || !cov) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
+  tscm_options defaults;
+  tscm_options_init(&defaults);
+  if (!options) options = &defaults;
+  RC_TRY(validate_options(options));
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+    cudaGetLastError();
+    set_error("no CUDA device: the covariance has no CPU fallback");
+    return TSCM_ERR_NO_DEVICE;
+  }
+  if (device < 0) CUDA_TRY(cudaGetDevice(&device));
+  const int ngpu = std::max(1, options->num_gpus);
+  // the solver cache of tscm_solve(): after a solve of this structure only data is uploaded
+  tscm_solver* s = cache_checkout(problem, device, ngpu);
+  int rc = TSCM_OK;
+  if (s) {
+    rc = tscm_solver_set_options(s, options);
+  } else {
+    tscm_problem q = *problem;
+    q.obs_xy = nullptr;
+    rc = tscm_solver_create(&q, options, device, &s);
+  }
+  if (!rc) rc = upload_all_observations(s, problem->obs_xy);
+  if (!rc) rc = tscm_solver_set_parameters(s, intrinsics, cam_rt, board_rt);
+  if (!rc) rc = tscm_solver_covariance(s, cov);
+  if (s) cache_checkin(s, device, ngpu, rc == TSCM_OK || rc == TSCM_ERR_RANK_DEFICIENT);
+  return rc;
 }
 
 int tscm_solver_time_stage(tscm_solver* s, int stage, int repeats, double* ms_per_launch) {

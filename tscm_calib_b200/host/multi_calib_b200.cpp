@@ -135,6 +135,71 @@ MultiCalib::MultiCalib(std::vector<TripleSphereCamera> cameras, const std::vecto
 }
 
 // Replaces multi_calib.cpp:155-284.
+bool MultiCalib::compute_covariance() {
+  const int C = (int)cameras_.size(), B = (int)chessboards_.size(), K = (int)worlds_.size();
+  std::vector<double> board_xy(2 * (size_t)K);
+  for (int j = 0; j < K; ++j) { board_xy[2 * j] = worlds_[j].x; board_xy[2 * j + 1] = worlds_[j].y; }
+  // the problem calibrate() solves: views (m, i) with an initialised board detected by camera m
+  std::vector<int> frame_id(B, -1);
+  std::vector<char> used(B, 0);
+  for (int m = 0; m < C; ++m) {
+    const auto& px = cameras_[m].pixels_ref();
+    for (int i = 0; i < B; ++i)
+      if (chessboards_[i].is_initial() && (int)px[i].size() == K) used[i] = 1;
+  }
+  int F = 0;
+  for (int i = 0; i < B; ++i) if (used[i]) frame_id[i] = F++;
+  std::vector<int32_t> view_camera, view_frame;
+  std::vector<double> obs;
+  for (int m = 0; m < C; ++m) {
+    const auto& px = cameras_[m].pixels_ref();
+    for (int i = 0; i < B; ++i) {
+      if (frame_id[i] < 0 || (int)px[i].size() != K) continue;
+      view_camera.push_back(m);
+      view_frame.push_back(frame_id[i]);
+      const double* d = reinterpret_cast<const double*>(px[i].data());   // cv::Point2d = {x, y}
+      obs.insert(obs.end(), d, d + 2 * (size_t)K);
+    }
+  }
+  if (F == 0 || view_camera.empty()) return false;
+  std::vector<double> intr(9 * (size_t)C), cam_rt(6 * (size_t)C), board_rt(6 * (size_t)F);
+  for (int m = 0; m < C; ++m) {
+    std::memcpy(&intr[9 * m], cameras_[m].intrinsic_.data(), sizeof(double) * 9);
+    std::memcpy(&cam_rt[6 * m], cameras_[m].rt_.data(), sizeof(double) * 6);
+  }
+  for (int i = 0; i < B; ++i)
+    if (frame_id[i] >= 0) std::memcpy(&board_rt[6 * frame_id[i]], chessboards_[i].rt_.data(), sizeof(double) * 6);
+  tscm_problem p;
+  p.num_cameras = C; p.num_frames = F; p.corners_per_board = K; p.num_views = (int)view_camera.size();
+  p.board_xy = board_xy.data(); p.view_camera = view_camera.data(); p.view_frame = view_frame.data();
+  p.obs_xy = obs.data();
+  p.fixed_camera = 0;
+  const int n = 6 * (C - 1) + 7 * C;
+  std::vector<double> cam_cov((size_t)n * n), board_cov(36 * (size_t)F);
+  tscm_covariance cov;
+  cov.camera = cam_cov.data(); cov.board = board_cov.data();
+  cov.residual_variance = 0.0; cov.kernel_ms = 0.0;
+  tscm_options opt = options_;
+  opt.verbose = 0;
+  const int rc = tscm_compute_covariance(&p, &opt, intr.data(), cam_rt.data(), board_rt.data(), &cov, device);
+  if (rc != TSCM_OK) {
+    if (!quiet) std::cout << "[tscm] covariance failed: " << tscm_last_error() << std::endl;
+    return false;
+  }
+  const double s2 = cov.residual_variance;
+  residual_variance = s2;
+  camera_std_dev.assign(C, std::vector<double>(15, 0.0));
+  int o = 0;
+  for (int m = 0; m < C; ++m) {
+    for (int k = (m == 0 ? 6 : 0); k < 13; ++k, ++o) camera_std_dev[m][k] = std::sqrt(s2 * cam_cov[(size_t)o * n + o]);
+  }
+  board_std_dev.assign(B, std::vector<double>(6, 0.0));
+  for (int i = 0; i < B; ++i)
+    if (frame_id[i] >= 0)
+      for (int k = 0; k < 6; ++k) board_std_dev[i][k] = std::sqrt(s2 * board_cov[36 * (size_t)frame_id[i] + 7 * k]);
+  return true;
+}
+
 void MultiCalib::calibrate() {
   const int C = (int)cameras_.size(), B = (int)chessboards_.size(), K = (int)worlds_.size();
   std::vector<double> board_xy(2 * (size_t)K);

@@ -76,6 +76,17 @@ class MultiCalib {
   void calibrate();
   // main.cpp:293-319.  Returns false when the file cannot be written.
   bool write_yaml(const std::string& filename);
+  // Parameter uncertainties at the current parameters (call it after calibrate()), through
+  // tscm_compute_covariance() with options() (so num_gpus applies): fills camera_std_dev and
+  // board_std_dev with sqrt(residual_variance * diag(Sigma)), OpenCV's stdDeviations.  Returns
+  // false (and leaves them untouched) when there is nothing to compute or the covariance fails,
+  // e.g. TSCM_ERR_RANK_DEFICIENT.
+  bool compute_covariance();
+  // C x 15: [rt 6 | fx fy cx cy xi lambda alpha b c]; 0 where not free (camera 0's rt, b, c)
+  std::vector<std::vector<double>> camera_std_dev;
+  // B x 6: board pose [angle-axis 3 | t 3]; 0 for boards that are not part of the problem
+  std::vector<std::vector<double>> board_std_dev;
+  double residual_variance = 0.0;
   std::vector<MultiCalib_camera> cameras_;
   std::vector<MultiCalib_chessboard> chessboards_;
   std::vector<cv::Point3d> worlds_;
