@@ -71,6 +71,12 @@ enum {
   TSCM_ERR_RANK_DEFICIENT = 7 /* covariance: H is singular (gauge freedom, degenerate board) */
 };
 
+/* Size limit: the reduced camera system has NL = 13 C - 6 live parameters (13 C with
+ * fixed_camera = -1), and it is factored in the shared memory of one thread block.  A solver
+ * accepts NL <= 202: at most 16 cameras with one fixed, or 15 with none (16 cameras with none
+ * fixed, NL 208, need 233,984 bytes per block, over the 232,448 of a B200).  Larger problems
+ * fail with TSCM_ERR_UNSUPPORTED at creation (tscm_solver_create, tscm_solve,
+ * tscm_compute_covariance). */
 typedef struct tscm_problem {
   int32_t num_cameras;        /* C  (cameras_.size(), multi_calib.cpp:157) */
   int32_t num_frames;         /* F  (chessboards_.size(), multi_calib.cpp:158); every frame

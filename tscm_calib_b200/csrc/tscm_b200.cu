@@ -845,8 +845,15 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   for (int c = 0; c < C; ++c) live_off[c + 1] = live_off[c] + (c == p->fixed_camera ? 7 : 13);
   const int NL = live_off[C];
   P.NL = NL; P.Q = NL * (NL + 1) / 2;
-  if (NL > 216) {
-    set_error("reduced system of %d live parameters exceeds this build's limit (216, i.e. 17 cameras)", NL);
+  // The reduced system is factored by ONE CTA of k_solve, and the covariance kernels size their
+  // shared arrays by kCovMaxNL: a system is accepted when both fit.  On a B200 (232,448 bytes of
+  // opt-in shared memory per block) k_solve is the tighter bound: 16 cameras with one fixed
+  // (NL 202) need 220,056 bytes, 16 with none fixed (NL 208) 233,984.
+  s->solve = solve_dims(NL, C);
+  if (NL > kCovMaxNL || s->solve.smem > s->smem_optin || cov_factor_smem(NL) > s->smem_optin) {
+    set_error("reduced system of %d live parameters (%d cameras) exceeds the limit of %d (16 cameras with one "
+              "fixed): the solve needs %zu bytes of shared memory per block, the device allows %zu",
+              NL, C, kCovMaxNL, s->solve.smem, s->smem_optin);
     free_shard(s); return TSCM_ERR_UNSUPPORTED;
   }
   std::vector<short> live_cam(NL), live_kk(NL);
@@ -911,11 +918,10 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   s->schur_nblk = (F + fpb - 1) / fpb;
   s->schur.frames_per_block = fpb;
   s->schur.Fpad = (F + 31) / 32 * 32;
-  s->solve = solve_dims(NL, C);
   s->eval5_smem = e5_smem_bytes(K, C);
-  if (s->eval5_smem > s->smem_optin || s->solve.smem > s->smem_optin) {
-    set_error("problem (%d corners, %d cameras) needs %zu / %zu bytes of shared memory per CTA (limit %zu)", K, C,
-              s->eval5_smem, s->solve.smem, s->smem_optin);
+  if (s->eval5_smem > s->smem_optin) {
+    set_error("problem (%d corners, %d cameras) needs %zu bytes of shared memory per CTA in k_eval5 (limit %zu)", K, C,
+              s->eval5_smem, s->smem_optin);
     free_shard(s); return TSCM_ERR_UNSUPPORTED;
   }
   lap("index tables (host)");
@@ -971,7 +977,9 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   {
     int maxv = 1;
     for (int f = 0; f < F; ++f) maxv = std::max(maxv, frame_ptr[f + 1] - frame_ptr[f]);
-    s->post_lpf = maxv <= 8 ? 8 : (maxv <= 16 ? 16 : 32);     // <= 17 cameras
+    // a frame has at most one view per camera, and the limit above admits at most 16 cameras:
+    // 32 lanes are reachable only if that limit is raised
+    s->post_lpf = maxv <= 8 ? 8 : (maxv <= 16 ? 16 : 32);
     const int fpc = kPostThreads / s->post_lpf;
     s->fg_nblk = (F + fpc - 1) / fpc;
   }
@@ -989,6 +997,13 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
     s->e5items = e5_items((int)ntile_e, std::min((int)ntile_e, s->sm_count), (K + kE5Producers - 1) / kE5Producers);
     A.want(&s->d_mom, (size_t)s->e5items.nitems * kE5MomEntries * 32);
     A.want(&s->d_fcg, ntile_e * kFcElems * 32);
+    if (g_debug & 1)
+      std::fprintf(stderr,
+                   "[tscm create] paths: form=%s ept=%d solveT=%d lpf=%d e5grid=%d e5tiles=%d e5whole=%d e5split=%d "
+                   "NL=%d solve_smem=%zu smem_optin=%zu\n",
+                   form == kSchurRows ? "rows" : (form == kSchurFused ? "fused" : "pairs"), s->schur_ept, s->solve.T,
+                   s->post_lpf, std::min((int)ntile_e, s->sm_count), (int)ntile_e, s->e5items.n_whole,
+                   s->e5items.split, NL, s->solve.smem, s->smem_optin);
   }
   const int cap = std::max(128, std::min(s->options.max_num_iterations, 1 << 16) + 2);
   A.want(&s->d_trace, trace_bytes(cap));

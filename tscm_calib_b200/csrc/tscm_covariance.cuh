@@ -4,7 +4,7 @@
 //   camera block   Sigma_cc = D_c S~^-1 D_c,               S~ = U~ - W~^T V~^-1 W~
 //   board block f  Sigma_ff = D_e,f (V~_f^-1 + Y~_f S~^-1 Y~_f^T) D_e,f,   Y~_f = V~_f^-1 W~_f
 // Three kernels:
-//   k_cov_factor   ONE CTA: the packed lower triangle of S~ (at most 216 live columns: 187 KB)
+//   k_cov_factor   ONE CTA: the packed lower triangle of S~ (at most 202 live columns: 164 KB)
 //                  in shared memory, right-looking LDL^T with one barrier per column and the
 //                  rank test of ceres::Covariance (pivot <= 1e-14 x largest diagonal entry);
 //                  the unit-lower factor goes to global memory mirrored into both triangles
@@ -24,7 +24,10 @@
 
 namespace tscm {
 
-constexpr int kCovMaxNL = 216;              // the largest reduced system a solver accepts
+// The largest reduced system a solver accepts (create_shard checks it with k_solve's shared memory,
+// solve_dims(), which is the tighter bound on a B200: 16 cameras with one fixed).  It sizes the
+// static shared arrays of k_cov_inverse and k_cov_frames.
+constexpr int kCovMaxNL = 202;
 constexpr int kCovFactorThreads = 512;
 constexpr int kCovInvWarps = 4;             // identity columns per CTA of k_cov_inverse
 constexpr int kCovFrameWarps = 4;           // frames per CTA of k_cov_frames
