@@ -72,11 +72,15 @@ enum {
 };
 
 /* Size limit: the reduced camera system has NL = 13 C - 6 live parameters (13 C with
- * fixed_camera = -1), and it is factored in the shared memory of one thread block.  A solver
- * accepts NL <= 202: at most 16 cameras with one fixed, or 15 with none (16 cameras with none
+ * fixed_camera = -1), and by default it is factored in the shared memory of one thread block.  A
+ * solver accepts NL <= 202: at most 16 cameras with one fixed, or 15 with none (16 cameras with none
  * fixed, NL 208, need 233,984 bytes per block, over the 232,448 of a B200).  Larger problems
  * fail with TSCM_ERR_UNSUPPORTED at creation (tscm_solver_create, tscm_solve,
- * tscm_compute_covariance). */
+ * tscm_compute_covariance).
+ * With tscm_options.allow_large_rigs = 1 the limit is NL <= 416 (32 cameras, with or without a
+ * fixed one): systems above 202 are factored by a thread-block cluster of 2-8 CTAs, and their
+ * covariance by a factor in global memory.  Sharded solves (num_gpus > 1, tscm_solver_attach_comm,
+ * tscm_solver_p2p_attach) stay limited to NL <= 202 and return TSCM_ERR_UNSUPPORTED above. */
 typedef struct tscm_problem {
   int32_t num_cameras;        /* C  (cameras_.size(), multi_calib.cpp:157) */
   int32_t num_frames;         /* F  (chessboards_.size(), multi_calib.cpp:158); every frame
@@ -123,6 +127,10 @@ typedef struct tscm_options {
                                                (SURVEY.md 8b/8e; peer access between them is required).
                                                The reference is single-process, so this is how
                                                MultiCalib::calibrate() reaches more than one GPU. */
+  int32_t allow_large_rigs;                 /* 0 (default): NL <= 202 (see "Size limit").  1: NL <= 416,
+                                               up to 32 cameras, one GPU above 202.  Fixed when the
+                                               solver is created: tscm_solver_set_options refuses a
+                                               change with TSCM_ERR_INVALID_ARGUMENT. */
 } tscm_options;
 
 typedef struct tscm_summary {
@@ -284,6 +292,10 @@ int tscm_solver_time_stage(tscm_solver* solver, int stage, int repeats, double* 
  * producer/consumer CTA (k_schur2), 3 = per-camera-pair (k_pair_* + k_schur_pairs2).  Returns
  * TSCM_ERR_UNSUPPORTED when the form cannot hold this problem. */
 int tscm_solver_set_schur_form(tscm_solver* solver, int form);
+/* Test hook: the kernel of the reduced solve.  0 = chosen from NL (what every production call
+ * uses: one CTA up to 202 live parameters, a thread-block cluster above), 1 = one CTA (k_solve;
+ * TSCM_ERR_UNSUPPORTED above 202), 2 = cluster (k_solve_cluster, at any size). */
+int tscm_solver_set_reduced_solve(tscm_solver* solver, int form);
 /* bit 0: creation / solve phase timings on stderr; bit 1: in-kernel cycle counts of k_solve;
  * bit 2: solvers created from now on chain their kernels WITHOUT programmatic dependent launch
  * (A/B timing). */

@@ -11,7 +11,7 @@ LIB = os.path.join(_HERE, "libtscm_b200.so")
 SOURCES = ["tscm_b200.cu", "tscm_monoinit.cu"]
 # per-source flags: the mono cold start mirrors scalar IEEE statements (no FMA contraction)
 SOURCE_FLAGS = {"tscm_monoinit.cu": ["-fmad=false"]}
-HEADERS = ["tscm_kernels.cuh", "tscm_eval5.cuh", "tscm_solve.cuh", "tscm_math.cuh", "tscm_p2p.cuh", "tscm_remap.cuh", "tscm_posegraph.cuh", "tscm_covariance.cuh", "tscm_internal.h", "tscm_schur_pairs.cuh", "tscm_pair_lists.h", os.path.join("..", "..", "include", "tscm.h")]
+HEADERS = ["tscm_kernels.cuh", "tscm_eval5.cuh", "tscm_solve.cuh", "tscm_solve_cluster.cuh", "tscm_math.cuh", "tscm_p2p.cuh", "tscm_remap.cuh", "tscm_posegraph.cuh", "tscm_covariance.cuh", "tscm_internal.h", "tscm_schur_pairs.cuh", "tscm_pair_lists.h", os.path.join("..", "..", "include", "tscm.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

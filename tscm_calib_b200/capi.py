@@ -56,6 +56,7 @@ class TscmOptions(C.Structure):
         ("disable_tolerances", C.c_int32),
         ("verbose", C.c_int32),
         ("num_gpus", C.c_int32),
+        ("allow_large_rigs", C.c_int32),
     ]
 
 
@@ -160,6 +161,7 @@ def default_options(**overrides) -> TscmOptions:
     o.disable_tolerances = 0
     o.verbose = 0
     o.num_gpus = 1
+    o.allow_large_rigs = 0
     for k, v in overrides.items():
         if k == "loss_type" and isinstance(v, str):
             v = LOSS[v]
@@ -294,6 +296,8 @@ def load_library(path: str | None = None):
     lib.tscm_solver_set_exchange_timeout.restype = C.c_int
     lib.tscm_solver_set_schur_form.argtypes = [C.c_void_p, C.c_int]
     lib.tscm_solver_set_schur_form.restype = C.c_int
+    lib.tscm_solver_set_reduced_solve.argtypes = [C.c_void_p, C.c_int]
+    lib.tscm_solver_set_reduced_solve.restype = C.c_int
     lib.tscm_set_debug.argtypes = [C.c_int32]
     lib.tscm_set_debug.restype = None
     lib.tscm_solver_create.argtypes = [P(TscmProblem), P(TscmOptions), C.c_int, P(C.c_void_p)]
@@ -364,12 +368,13 @@ EXPORTED_SYMBOLS = [
     "tscm_last_error", "tscm_version", "tscm_cache_configure", "tscm_cache_release",
     "tscm_host_alloc", "tscm_host_free", "tscm_solver_set_exchange_timeout",
     "tscm_solver_set_schur_form", "tscm_set_debug", "tscm_pose_graph_init", "tscm_mono_init",
-    "tscm_solver_covariance", "tscm_compute_covariance",
+    "tscm_solver_covariance", "tscm_compute_covariance", "tscm_solver_set_reduced_solve",
 ]
 
 ERR_RANK_DEFICIENT = 7   # TSCM_ERR_RANK_DEFICIENT
 
 SCHUR_FORM = {"auto": 0, "rows": 1, "fused": 2, "pairs": 3}
+REDUCED_SOLVE = {"auto": 0, "single": 1, "cluster": 2}
 
 
 class TscmError(RuntimeError):
@@ -444,6 +449,11 @@ class Solver:
         """Test hook (tscm_solver_set_schur_form): 'auto' | 'rows' | 'fused' | 'pairs'."""
         f = SCHUR_FORM[form] if isinstance(form, str) else int(form)
         check(self.lib.tscm_solver_set_schur_form(self.h, f), self.lib)
+
+    def set_reduced_solve(self, form):
+        """Test hook (tscm_solver_set_reduced_solve): 'auto' | 'single' | 'cluster'."""
+        f = REDUCED_SOLVE[form] if isinstance(form, str) else int(form)
+        check(self.lib.tscm_solver_set_reduced_solve(self.h, f), self.lib)
 
     def set_exchange_timeout(self, seconds: float):
         check(self.lib.tscm_solver_set_exchange_timeout(self.h, float(seconds)), self.lib)

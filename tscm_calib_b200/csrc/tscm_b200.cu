@@ -33,6 +33,7 @@
 #include "tscm_kernels.cuh"
 #include "tscm_eval5.cuh"
 #include "tscm_solve.cuh"
+#include "tscm_solve_cluster.cuh"
 #include "tscm_p2p.cuh"
 #include "tscm_schur_pairs.cuh"
 #include "tscm_pair_lists.h"
@@ -238,6 +239,10 @@ struct tscm_solver {
   int schur2_nt = 0;
   int schur_nblk = 0, schur_nt = 256, schur_ept = 1;
   SolveDims solve{};
+  // reduced solve (tscm_solve_cluster.cuh): single CTA up to kCovMaxNL live parameters, cluster above
+  bool use_cluster = false;         // the form in use (tscm_solver_set_reduced_solve forces one)
+  ClusterDims cluster{};
+  double* d_cluster_L = nullptr;    // [solve_pan_off(nbk, nbk)] factor panels of k_solve_cluster
   size_t eval5_smem = 0;
   E5Items e5items{};
   int want_err = 0;                 // accumulate sum sqrt(s) (reprojection read-out only)
@@ -278,6 +283,7 @@ struct tscm_solver {
   double* d_cov_sinv = nullptr;     // [NL][NL] S~^-1 (scaled)
   double* d_cov_cam = nullptr;      // [NL][NL] camera block, unscaled
   double* d_cov_board = nullptr;    // [F][36] board blocks, unscaled
+  double* d_cov_tri = nullptr;      // packed lower triangle of S~ for the factor above kCovMaxNL
   int* d_cov_flag = nullptr;
   cudaEvent_t cov_ev[2] = {nullptr, nullptr};
 };
@@ -318,9 +324,28 @@ bool lm_equal(const LmOptions& a, const LmOptions& b) {
 int validate_options(const tscm_options* o) {
   if (o->max_num_iterations < 0 || !(o->initial_trust_region_radius > 0.0) ||
       (o->loss_type != TSCM_LOSS_NONE && !(o->loss_scale > 0.0)) || o->loss_type < 0 ||
-      o->loss_type > TSCM_LOSS_CAUCHY || o->num_gpus < 0 || o->num_gpus > kP2PMaxRanks) {
+      o->loss_type > TSCM_LOSS_CAUCHY || o->num_gpus < 0 || o->num_gpus > kP2PMaxRanks ||
+      (o->allow_large_rigs != 0 && o->allow_large_rigs != 1)) {
     set_error("invalid options");
     return TSCM_ERR_INVALID_ARGUMENT;
+  }
+  return TSCM_OK;
+}
+
+// The limits of the opt-in to reduced systems wider than one CTA holds, from the host tables alone
+// (before any device is touched).  Without the opt-in create_shard applies the default limit.
+int validate_large_rig(const tscm_problem* p, const tscm_options* o) {
+  if (!o->allow_large_rigs) return TSCM_OK;
+  const int NL = 13 * p->num_cameras - (p->fixed_camera >= 0 ? 6 : 0);
+  if (NL > kLargeRigMaxNL) {
+    set_error("reduced system of %d live parameters (%d cameras) exceeds the limit of %d of allow_large_rigs "
+              "(32 cameras with none fixed)", NL, p->num_cameras, kLargeRigMaxNL);
+    return TSCM_ERR_UNSUPPORTED;
+  }
+  if (NL > kCovMaxNL && o->num_gpus > 1) {
+    set_error("reduced system of %d live parameters: sharded solves (num_gpus > 1) support at most %d", NL,
+              kCovMaxNL);
+    return TSCM_ERR_UNSUPPORTED;
   }
   return TSCM_OK;
 }
@@ -493,7 +518,27 @@ int launch_schur_allreduce(tscm_solver* s, double radius_override) {
   return TSCM_OK;
 }
 
+// k_solve_cluster: a cluster of ncta CTAs, with programmatic dependent launch like every kernel
+void launch_solve_cluster(tscm_solver* s) {
+  const ClusterDims& d = s->cluster;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(d.ncta); cfg.blockDim = dim3(kClusterThreads); cfg.dynamicSmemBytes = d.smem;
+  cfg.stream = s->stream;
+  cudaLaunchAttribute attr[2];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = d.ncta; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = s->pdl ? 2 : 1;
+  auto kernel = s->P.NL <= 32 * 7 ? k_solve_cluster<7> : k_solve_cluster<13>;
+  cudaLaunchKernelEx(&cfg, kernel, s->P, s->ps[0], s->ps[1], s->d_state, (const double*)s->d_Sr,
+                     (const double*)s->d_scale_c, s->d_yc, s->d_cluster_L, d.tpc, d.tail_nt);
+  s->launches += 1;
+}
+
 void launch_solve(tscm_solver* s) {
+  if (s->use_cluster) { launch_solve_cluster(s); return; }
   const SolveDims& d = s->solve;
   const int prof = (g_debug & 2) ? 1 : 0;
   if (d.T == 1)
@@ -745,6 +790,56 @@ int set_smem_attr(const void* fn, size_t bytes) {
   return TSCM_OK;
 }
 
+// Whether the single-CTA k_solve (and the shared-memory k_cov_factor) hold this solver's reduced
+// system: the default limit, and the choice between k_solve and k_solve_cluster.  Needs s->solve.
+bool single_cta_fits(const tscm_solver* s) {
+  const int NL = s->P.NL;
+  return NL <= kCovMaxNL && s->solve.smem <= s->smem_optin && cov_factor_smem(NL) <= s->smem_optin;
+}
+
+// Prepares k_solve_cluster for this solver: cluster size, the global copy of the factor, and a
+// check that the device can schedule the cluster with its shared memory (so that no launch inside
+// the iteration graph can fail for it).
+int ensure_cluster(tscm_solver* s) {
+  if (s->d_cluster_L) return TSCM_OK;
+  const int NL = s->P.NL;
+  const ClusterDims d = cluster_dims(NL, s->C);
+  if (NL > kLargeRigMaxNL || d.ncta > kClusterMaxCtas) {
+    set_error("reduced system of %d live parameters exceeds the limit of %d of the cluster solve", NL, kLargeRigMaxNL);
+    return TSCM_ERR_UNSUPPORTED;
+  }
+  // the attribute is per kernel and process-wide: set it once to the largest system accepted
+  // (32 cameras, 416 live parameters), so that a solver never lowers it under another's launch
+  const size_t smem_max = cluster_dims(kLargeRigMaxNL, 32).smem;
+  if (d.smem > smem_max || smem_max > s->smem_optin) {
+    set_error("cluster solve needs %zu bytes of shared memory per block, the device allows %zu", smem_max, s->smem_optin);
+    return TSCM_ERR_UNSUPPORTED;
+  }
+  const void* fns[2] = {(const void*)k_solve_cluster<7>, (const void*)k_solve_cluster<13>};
+  const void* fn = NL <= 32 * 7 ? fns[0] : fns[1];
+  for (const void* f : fns) CUDA_TRY(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(d.ncta); cfg.blockDim = dim3(kClusterThreads); cfg.dynamicSmemBytes = d.smem;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = d.ncta; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  int nclusters = 0;
+  const cudaError_t e = cudaOccupancyMaxActiveClusters(&nclusters, fn, &cfg);
+  if (e != cudaSuccess || nclusters < 1) {
+    cudaGetLastError();
+    set_error("the device cannot schedule a cluster of %d CTAs with %zu bytes of shared memory each (%s)", d.ncta,
+              d.smem, e != cudaSuccess ? cudaGetErrorString(e) : "no active cluster");
+    return TSCM_ERR_UNSUPPORTED;
+  }
+  double* L = nullptr;
+  CUDA_TRY(cudaMalloc((void**)&L, (size_t)solve_pan_off(d.nbk, d.nbk) * sizeof(double)));
+  s->extra.push_back(L);
+  s->d_cluster_L = L;
+  s->cluster = d;
+  return TSCM_OK;
+}
+
 // after commit + upload
 int wire_schur(tscm_solver* s, int form) {
   s->split.col_ptr = s->schur2.col_ptr; s->split.col_src = s->schur2.col_src; s->split.col_g = s->schur2.col_g;
@@ -848,9 +943,13 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   // The reduced system is factored by ONE CTA of k_solve, and the covariance kernels size their
   // shared arrays by kCovMaxNL: a system is accepted when both fit.  On a B200 (232,448 bytes of
   // opt-in shared memory per block) k_solve is the tighter bound: 16 cameras with one fixed
-  // (NL 202) need 220,056 bytes, 16 with none fixed (NL 208) 233,984.
+  // (NL 202) need 220,056 bytes, 16 with none fixed (NL 208) 233,984.  With allow_large_rigs a
+  // wider system (up to kLargeRigMaxNL, validate_large_rig) goes to k_solve_cluster instead.
   s->solve = solve_dims(NL, C);
-  if (NL > kCovMaxNL || s->solve.smem > s->smem_optin || cov_factor_smem(NL) > s->smem_optin) {
+  const bool single_fits = single_cta_fits(s);
+  if (!single_fits && o->allow_large_rigs && !is_kid) {
+    s->use_cluster = true;
+  } else if (!single_fits) {
     set_error("reduced system of %d live parameters (%d cameras) exceeds the limit of %d (16 cameras with one "
               "fixed): the solve needs %zu bytes of shared memory per block, the device allows %zu",
               NL, C, kCovMaxNL, s->solve.smem, s->smem_optin);
@@ -977,8 +1076,7 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   {
     int maxv = 1;
     for (int f = 0; f < F; ++f) maxv = std::max(maxv, frame_ptr[f + 1] - frame_ptr[f]);
-    // a frame has at most one view per camera, and the limit above admits at most 16 cameras:
-    // 32 lanes are reachable only if that limit is raised
+    // a frame has at most one view per camera: 16 cameras by default, 32 with allow_large_rigs
     s->post_lpf = maxv <= 8 ? 8 : (maxv <= 16 ? 16 : 32);
     const int fpc = kPostThreads / s->post_lpf;
     s->fg_nblk = (F + fpc - 1) / fpc;
@@ -997,13 +1095,18 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
     s->e5items = e5_items((int)ntile_e, std::min((int)ntile_e, s->sm_count), (K + kE5Producers - 1) / kE5Producers);
     A.want(&s->d_mom, (size_t)s->e5items.nitems * kE5MomEntries * 32);
     A.want(&s->d_fcg, ntile_e * kFcElems * 32);
-    if (g_debug & 1)
+    if (g_debug & 1) {
+      // solveT / solve_smem: tiles per thread and shared memory per CTA of the kernel that runs;
+      // cluster: its CTAs (0: the single-CTA k_solve)
+      const ClusterDims cd = cluster_dims(NL, C);
       std::fprintf(stderr,
                    "[tscm create] paths: form=%s ept=%d solveT=%d lpf=%d e5grid=%d e5tiles=%d e5whole=%d e5split=%d "
-                   "NL=%d solve_smem=%zu smem_optin=%zu\n",
-                   form == kSchurRows ? "rows" : (form == kSchurFused ? "fused" : "pairs"), s->schur_ept, s->solve.T,
-                   s->post_lpf, std::min((int)ntile_e, s->sm_count), (int)ntile_e, s->e5items.n_whole,
-                   s->e5items.split, NL, s->solve.smem, s->smem_optin);
+                   "NL=%d solve_smem=%zu smem_optin=%zu cluster=%d\n",
+                   form == kSchurRows ? "rows" : (form == kSchurFused ? "fused" : "pairs"), s->schur_ept,
+                   s->use_cluster ? kClusterT : s->solve.T, s->post_lpf, std::min((int)ntile_e, s->sm_count),
+                   (int)ntile_e, s->e5items.n_whole, s->e5items.split, NL, s->use_cluster ? cd.smem : s->solve.smem,
+                   s->smem_optin, s->use_cluster ? cd.ncta : 0);
+    }
   }
   const int cap = std::max(128, std::min(s->options.max_num_iterations, 1 << 16) + 2);
   A.want(&s->d_trace, trace_bytes(cap));
@@ -1036,8 +1139,12 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
     s->p2p.timeout_ns = 10ull * 1000000000ull;
   }
   TRY_S(wire_schur(s, form));
-  TRY_S(set_smem_attr((const void*)k_solve<1, 4>, s->solve.smem));
-  TRY_S(set_smem_attr((const void*)k_solve<4, 7>, s->solve.smem));
+  if (s->use_cluster) {
+    TRY_S(ensure_cluster(s));
+  } else {
+    TRY_S(set_smem_attr((const void*)k_solve<1, 4>, s->solve.smem));
+    TRY_S(set_smem_attr((const void*)k_solve<4, 7>, s->solve.smem));
+  }
   TRY_S(set_smem_attr((const void*)k_eval5, s->eval5_smem));
   TRY_S(set_smem_attr((const void*)k_view_blocks, vb_smem_bytes()));
   lap("kernel attributes");
@@ -1242,11 +1349,12 @@ int upload_all_observations(tscm_solver* s, const double* obs_xy) {
 
 // The cached solver of this structure, taken out of the cache (nobody else may use it meanwhile),
 // or nullptr.
-tscm_solver* cache_checkout(const tscm_problem* p, int device, int ngpu) {
+tscm_solver* cache_checkout(const tscm_problem* p, int device, int ngpu, int allow_large_rigs) {
   std::lock_guard<std::mutex> lock(g_cache_mu);
   for (size_t i = 0; i < g_cache.size(); ++i) {
     CacheEntry& e = g_cache[i];
-    if (e.device == device && e.num_gpus == ngpu && same_structure(e.solver, p)) {
+    if (e.device == device && e.num_gpus == ngpu && e.solver->options.allow_large_rigs == allow_large_rigs &&
+        same_structure(e.solver, p)) {
       tscm_solver* s = e.solver;
       g_cache.erase(g_cache.begin() + i);
       return s;
@@ -1273,17 +1381,21 @@ void cache_checkin(tscm_solver* s, int device, int ngpu, bool keep) {
 int ensure_cov_buffers(tscm_solver* k) {
   if (k->d_cov_fac) return TSCM_OK;
   const size_t NL = (size_t)k->P.NL;
-  if (k->P.NL > kCovMaxNL) { set_error("covariance: %d live parameters exceed %d", k->P.NL, kCovMaxNL); return TSCM_ERR_UNSUPPORTED; }
-  if (cov_factor_smem(k->P.NL) > k->smem_optin) { set_error("covariance needs %zu bytes of shared memory", cov_factor_smem(k->P.NL)); return TSCM_ERR_UNSUPPORTED; }
+  // above kCovMaxNL (allow_large_rigs only) the factor works on a packed triangle in global memory
+  const bool large = k->P.NL > kCovMaxNL;
+  if (large && (!k->options.allow_large_rigs || k->P.NL > kLargeRigMaxNL)) { set_error("covariance: %d live parameters exceed %d", k->P.NL, kCovMaxNL); return TSCM_ERR_UNSUPPORTED; }
+  if (!large && cov_factor_smem(k->P.NL) > k->smem_optin) { set_error("covariance needs %zu bytes of shared memory", cov_factor_smem(k->P.NL)); return TSCM_ERR_UNSUPPORTED; }
   Arena a;
   a.want(&k->d_cov_fac, NL * NL);
   a.want(&k->d_cov_sinv, NL * NL);
   a.want(&k->d_cov_cam, NL * NL);
   a.want(&k->d_cov_board, (size_t)k->F * 36);
   a.want(&k->d_cov_flag, 1);
+  if (large) a.want(&k->d_cov_tri, NL * (NL + 1) / 2);
   RC_TRY(a.commit(k->stream));
   k->extra.push_back(a.base);
-  RC_TRY(set_smem_attr((const void*)k_cov_factor, cov_factor_smem(k->P.NL)));
+  if (!large) RC_TRY(set_smem_attr((const void*)k_cov_factor, cov_factor_smem(k->P.NL)));
+  RC_TRY(set_smem_attr((const void*)k_cov_frames, cov_frames_smem(kLargeRigMaxNL)));
   for (int e = 0; e < 2; ++e) CUDA_TRY(cudaEventCreate(&k->cov_ev[e]));
   return TSCM_OK;
 }
@@ -1293,11 +1405,15 @@ int launch_covariance(tscm_solver* k) {
   const int NL = k->P.NL, cur = k->x_in_set1 ? 1 : 0;
   CUDA_TRY(cudaMemsetAsync(k->d_cov_flag, 0, sizeof(int), k->stream));
   CUDA_TRY(cudaEventRecord(k->cov_ev[0], k->stream));
-  k_cov_factor<<<1, kCovFactorThreads, cov_factor_smem(NL), k->stream>>>(NL, k->solve.nbk, k->d_Sr, k->d_cov_fac,
-                                                                          k->d_cov_flag);
-  k_cov_inverse<<<(NL + kCovInvWarps - 1) / kCovInvWarps, 32 * kCovInvWarps, 0, k->stream>>>(
+  if (k->d_cov_tri)
+    k_cov_factor_global<<<1, kCovFactorThreads, 0, k->stream>>>(NL, k->solve.nbk, k->d_Sr, k->d_cov_fac,
+                                                                 k->d_cov_flag, k->d_cov_tri);
+  else
+    k_cov_factor<<<1, kCovFactorThreads, cov_factor_smem(NL), k->stream>>>(NL, k->solve.nbk, k->d_Sr, k->d_cov_fac,
+                                                                            k->d_cov_flag);
+  k_cov_inverse<<<(NL + kCovInvWarps - 1) / kCovInvWarps, 32 * kCovInvWarps, cov_inverse_smem(NL), k->stream>>>(
       k->P, k->d_scale_c, k->d_cov_fac, k->d_cov_flag, k->d_cov_sinv, k->d_cov_cam);
-  k_cov_frames<<<(k->F + kCovFrameWarps - 1) / kCovFrameWarps, 32 * kCovFrameWarps, 0, k->stream>>>(
+  k_cov_frames<<<(k->F + kCovFrameWarps - 1) / kCovFrameWarps, 32 * kCovFrameWarps, cov_frames_smem(NL), k->stream>>>(
       k->P, k->ps[cur], k->d_scale_e, k->d_scale_c, k->schur.frame_rec, k->schur.Fpad, k->d_cov_sinv, k->d_cov_flag,
       k->d_cov_board);
   CUDA_TRY(cudaEventRecord(k->cov_ev[1], k->stream));
@@ -1407,6 +1523,10 @@ void tscm_host_free(void* p) {
 int tscm_solver_set_options(tscm_solver* s, const tscm_options* o) {
   if (!s || !o) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   RC_TRY(validate_options(o));
+  if (o->allow_large_rigs != s->options.allow_large_rigs) {
+    set_error("allow_large_rigs is fixed when the solver is created");
+    return TSCM_ERR_INVALID_ARGUMENT;
+  }
   s->options = *o;
   return for_shards(s, [&](tscm_solver* k, int) -> int {
     LmOptions lm{};
@@ -1429,6 +1549,7 @@ int tscm_solver_create(const tscm_problem* p, const tscm_options* o, int device,
   tscm_options_init(&defaults);
   if (!o) o = &defaults;
   RC_TRY(validate_options(o));
+  RC_TRY(validate_large_rig(p, o));
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     cudaGetLastError();
@@ -1612,6 +1733,7 @@ int tscm_solve(const tscm_problem* problem, const tscm_options* options, double*
   tscm_options_init(&defaults);
   if (!options) options = &defaults;
   RC_TRY(validate_options(options));
+  RC_TRY(validate_large_rig(problem, options));
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     cudaGetLastError();
@@ -1621,7 +1743,7 @@ int tscm_solve(const tscm_problem* problem, const tscm_options* options, double*
   if (device < 0) CUDA_TRY(cudaGetDevice(&device));
   const int ngpu = std::max(1, options->num_gpus);
   // ---- solver: cached for this structure, or new ---------------------------------------------
-  tscm_solver* s = cache_checkout(problem, device, ngpu);
+  tscm_solver* s = cache_checkout(problem, device, ngpu, options->allow_large_rigs);
   const bool hit = s != nullptr;
   const double ms_lookup = ms_since(t0);
   int rc = TSCM_OK;
@@ -1667,10 +1789,18 @@ int tscm_comm_unique_id(void* unique_id_128) {
     }                                                                                               \
   } while (0)
 
+// Sharded solves exchange the reduced system at the default size limit only.
+static int no_large_shards(const tscm_solver* s) {
+  if (s->P.NL <= kCovMaxNL) return TSCM_OK;
+  set_error("reduced system of %d live parameters: multi-process solves support at most %d", s->P.NL, kCovMaxNL);
+  return TSCM_ERR_UNSUPPORTED;
+}
+
 int tscm_solver_attach_comm(tscm_solver* s, int rank, int num_ranks, const void* unique_id_128) {
   DeviceGuard device_guard_;
   if (!s || !unique_id_128 || rank < 0 || rank >= num_ranks) { set_error("bad comm arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_attach_comm");
+  RC_TRY(no_large_shards(s));
   NcclApi& n = nccl();
   if (!n.ok) { set_error("libnccl.so.2 could not be loaded"); return TSCM_ERR_COMM; }
   CUDA_TRY(cudaSetDevice(s->device));
@@ -1700,6 +1830,7 @@ int tscm_solver_p2p_attach(tscm_solver* s, int rank, int num_ranks, const void* 
   DeviceGuard device_guard_;
   if (!s || !handles || rank < 0 || rank >= num_ranks) { set_error("bad p2p arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_p2p_attach");
+  RC_TRY(no_large_shards(s));
   if (num_ranks > kP2PMaxRanks) { set_error("peer-memory exchange supports at most %d ranks", kP2PMaxRanks); return TSCM_ERR_INVALID_ARGUMENT; }
   CUDA_TRY(cudaSetDevice(s->device));
   for (int r = 0; r < num_ranks; ++r) {
@@ -1749,6 +1880,31 @@ int tscm_solver_set_schur_form(tscm_solver* s, int form) {
     b.d_base = d_blob;
     RC_TRY(b.upload(k->stream));
     return wire_schur(k, f);
+  });
+}
+
+int tscm_solver_set_reduced_solve(tscm_solver* s, int form) {
+  DeviceGuard device_guard_;
+  if (!s || form < 0 || form > 2) { set_error("bad arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
+  return for_shards(s, [&](tscm_solver* k, int) -> int {
+    CUDA_TRY(cudaSetDevice(k->device));
+    const bool fits = single_cta_fits(k);
+    const bool cluster = form == 2 || (form == 0 && !fits);
+    if (!cluster && !fits) {
+      set_error("the single-CTA solve cannot hold a reduced system of %d live parameters (limit %d)", k->P.NL,
+                kCovMaxNL);
+      return TSCM_ERR_UNSUPPORTED;
+    }
+    if (cluster) {
+      CUDA_TRY(cudaStreamSynchronize(k->stream));
+      RC_TRY(ensure_cluster(k));
+    } else {
+      RC_TRY(set_smem_attr((const void*)k_solve<1, 4>, k->solve.smem));
+      RC_TRY(set_smem_attr((const void*)k_solve<4, 7>, k->solve.smem));
+    }
+    k->use_cluster = cluster;
+    k->graph_dirty = true;
+    return TSCM_OK;
   });
 }
 
@@ -1983,6 +2139,7 @@ int tscm_compute_covariance(const tscm_problem* problem, const tscm_options* opt
   tscm_options_init(&defaults);
   if (!options) options = &defaults;
   RC_TRY(validate_options(options));
+  RC_TRY(validate_large_rig(problem, options));
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     cudaGetLastError();
@@ -1992,7 +2149,7 @@ int tscm_compute_covariance(const tscm_problem* problem, const tscm_options* opt
   if (device < 0) CUDA_TRY(cudaGetDevice(&device));
   const int ngpu = std::max(1, options->num_gpus);
   // the solver cache of tscm_solve(): after a solve of this structure only data is uploaded
-  tscm_solver* s = cache_checkout(problem, device, ngpu);
+  tscm_solver* s = cache_checkout(problem, device, ngpu, options->allow_large_rigs);
   int rc = TSCM_OK;
   if (s) {
     rc = tscm_solver_set_options(s, options);

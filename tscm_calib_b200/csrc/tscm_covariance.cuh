@@ -5,7 +5,10 @@
 //   board block f  Sigma_ff = D_e,f (V~_f^-1 + Y~_f S~^-1 Y~_f^T) D_e,f,   Y~_f = V~_f^-1 W~_f
 // Three kernels:
 //   k_cov_factor   ONE CTA: the packed lower triangle of S~ (at most 202 live columns: 164 KB)
-//                  in shared memory, right-looking LDL^T with one barrier per column and the
+//                  in shared memory (k_cov_factor_global: the same code on a triangle in global
+//                  memory, for the wider systems of allow_large_rigs, up to 416 columns: 678 KB,
+//                  L2-resident; it runs once per covariance call, so simplicity beats speed),
+//                  right-looking LDL^T with one barrier per column and the
 //                  rank test of ceres::Covariance (pivot <= 1e-14 x largest diagonal entry);
 //                  the unit-lower factor goes to global memory mirrored into both triangles
 //                  (row i holds L[i][k<i] and L[k>i][i]) with 1/d on the diagonal, so that the
@@ -24,9 +27,9 @@
 
 namespace tscm {
 
-// The largest reduced system a solver accepts (create_shard checks it with k_solve's shared memory,
-// solve_dims(), which is the tighter bound on a B200: 16 cameras with one fixed).  It sizes the
-// static shared arrays of k_cov_inverse and k_cov_frames.
+// The largest reduced system a solver accepts by default (create_shard checks it with k_solve's
+// shared memory, solve_dims(), which is the tighter bound on a B200: 16 cameras with one fixed),
+// and the largest that k_cov_factor holds in shared memory.
 constexpr int kCovMaxNL = 202;
 constexpr int kCovFactorThreads = 512;
 constexpr int kCovInvWarps = 4;             // identity columns per CTA of k_cov_inverse
@@ -34,11 +37,14 @@ constexpr int kCovFrameWarps = 4;           // frames per CTA of k_cov_frames
 constexpr double kCovMinRcond = 1e-14;      // ceres::Covariance::Options::min_reciprocal_condition_number
 
 __host__ __device__ inline size_t cov_factor_smem(int NL) { return (size_t)NL * (NL + 1) / 2 * sizeof(double); }
+// dynamic shared memory of k_cov_inverse (x per warp) and k_cov_frames (W~_f and its columns per warp)
+inline size_t cov_inverse_smem(int NL) { return (size_t)kCovInvWarps * NL * sizeof(double); }
+inline size_t cov_frames_smem(int NL) { return (size_t)kCovFrameWarps * NL * (6 * sizeof(double) + sizeof(short)); }
 
 // flag bits: 1 = S~ is rank deficient, 2 = some V~_f is
-__global__ void __launch_bounds__(kCovFactorThreads)
-k_cov_factor(int NL, int nbk, const double* __restrict__ Sr, double* __restrict__ fac, int* __restrict__ flag) {
-  extern __shared__ double a[];               // row i at i (i + 1) / 2
+// a: the packed lower triangle, row i at i (i + 1) / 2, in shared or global memory of this CTA.
+__device__ __forceinline__ void cov_ldlt(double* a, int NL, int nbk, const double* __restrict__ Sr,
+                                         double* __restrict__ fac, int* __restrict__ flag) {
   __shared__ double s_thr;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
   for (int i = warp; i < NL; i += nw)
@@ -83,6 +89,19 @@ k_cov_factor(int NL, int nbk, const double* __restrict__ Sr, double* __restrict_
   }
 }
 
+__global__ void __launch_bounds__(kCovFactorThreads)
+k_cov_factor(int NL, int nbk, const double* __restrict__ Sr, double* __restrict__ fac, int* __restrict__ flag) {
+  extern __shared__ double a[];
+  cov_ldlt(a, NL, nbk, Sr, fac, flag);
+}
+
+// tri: [NL (NL + 1) / 2] scratch
+__global__ void __launch_bounds__(kCovFactorThreads)
+k_cov_factor_global(int NL, int nbk, const double* __restrict__ Sr, double* __restrict__ fac, int* __restrict__ flag,
+                    double* tri) {
+  cov_ldlt(tri, NL, nbk, Sr, fac, flag);
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -93,12 +112,12 @@ __device__ __forceinline__ double warp_sum(double v) {
 __global__ void __launch_bounds__(32 * kCovInvWarps)
 k_cov_inverse(DeviceProblem P, const double* __restrict__ scale_c, const double* __restrict__ fac,
               const int* __restrict__ flag, double* __restrict__ Sinv, double* __restrict__ cam_out) {
-  __shared__ double s_x[kCovInvWarps][kCovMaxNL];
+  extern __shared__ double s_x[];             // [kCovInvWarps][NL]
   if (*flag) return;
   const int NL = P.NL, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int c = blockIdx.x * kCovInvWarps + warp;
   if (c >= NL) return;
-  double* x = s_x[warp];
+  double* x = s_x + warp * NL;
   for (int i = lane; i < NL; i += 32) x[i] = 0.0;
   __syncwarp();
   // forward: y_c = 1, y_i = -sum_{c <= k < i} L[i][k] y_k; then z = D^-1 y
@@ -162,8 +181,8 @@ __global__ void __launch_bounds__(32 * kCovFrameWarps)
 k_cov_frames(DeviceProblem P, ParamSet ps, const double* __restrict__ scale_e, const double* __restrict__ scale_c,
              const double* __restrict__ frame_rec, int Fpad, const double* __restrict__ Sinv,
              int* __restrict__ flag, double* __restrict__ out) {
-  __shared__ double s_w[kCovFrameWarps][kCovMaxNL][6];   // W~_f, one row per live column of the frame
-  __shared__ short s_g[kCovFrameWarps][kCovMaxNL];       // its live column in S~
+  extern __shared__ double s_w[];             // [kCovFrameWarps][NL][6] W~_f, one row per live column of
+                                              // the frame | [kCovFrameWarps][NL] its live column in S~
   if (*flag & 1) return;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int f = blockIdx.x * kCovFrameWarps + warp;
@@ -214,8 +233,8 @@ k_cov_frames(DeviceProblem P, ParamSet ps, const double* __restrict__ scale_e, c
     return;
   }
   // W~_f = D_e W D_c over the live columns of the cameras that see the frame
-  double (*W)[6] = s_w[warp];
-  short* g = s_g[warp];
+  double (*W)[6] = reinterpret_cast<double (*)[6]>(s_w + (size_t)warp * NL * 6);
+  short* g = reinterpret_cast<short*>(s_w + (size_t)kCovFrameWarps * NL * 6) + warp * NL;
   int nf = 0;
   for (int q = P.frame_ptr[f]; q < P.frame_ptr[f + 1]; ++q) {
     const int v = P.frame_views[q], m = P.view_camera[v];
