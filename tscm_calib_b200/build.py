@@ -8,7 +8,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB = os.path.join(_HERE, "libtscm_b200.so")
-SOURCES = ["tscm_b200.cu", "tscm_monoinit.cu"]
+SOURCES = ["tscm_b200.cu", "tscm_remap.cu", "tscm_posegraph.cu", "tscm_monoinit.cu"]
 # per-source flags: the mono cold start mirrors scalar IEEE statements (no FMA contraction)
 SOURCE_FLAGS = {"tscm_monoinit.cu": ["-fmad=false"]}
 HEADERS = ["tscm_kernels.cuh", "tscm_eval5.cuh", "tscm_solve.cuh", "tscm_solve_cluster.cuh", "tscm_math.cuh", "tscm_p2p.cuh", "tscm_remap.cuh", "tscm_posegraph.cuh", "tscm_covariance.cuh", "tscm_internal.h", "tscm_schur_pairs.cuh", "tscm_pair_lists.h", os.path.join("..", "..", "include", "tscm.h")]

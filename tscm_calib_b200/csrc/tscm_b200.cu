@@ -1,9 +1,13 @@
-// tscm_b200.cu — C-ABI implementation (include/tscm.h) and host orchestration
+// tscm_b200.cu — C-ABI implementation (include/tscm.h) of the solver and host orchestration
 // of the device-side Levenberg-Marquardt loop.  The host never touches a
 // residual: it uploads the problem, captures one LM iteration as a CUDA graph,
 // replays it, and reads back the summary.  There is no CPU fallback.
 //
 // Replaces: ceres::Solve at /root/reference/TS.cpp:278 and multi_calib.cpp:216.
+//
+// Besides the solver this file holds the error text, the device check and the device scope that
+// every translation unit shares (tscm_internal.h).  The remap tables (tscm_remap.cu), the pose
+// graph (tscm_posegraph.cu) and the mono cold start (tscm_monoinit.cu) have their own files.
 //
 // Host-side structure:
 //   * one tscm_solver per device ("shard"): every buffer lives in ONE arena allocation, every
@@ -37,38 +41,15 @@
 #include "tscm_p2p.cuh"
 #include "tscm_schur_pairs.cuh"
 #include "tscm_pair_lists.h"
-#include "tscm_remap.cuh"
-#include "tscm_posegraph.cuh"
 #include "tscm_covariance.cuh"
 #include "tscm_internal.h"
+
+using tscm::internal::set_error;
 
 namespace {
 
 thread_local std::string g_last_error;
 int g_debug = 0;     // tscm_set_debug(): bit 0 phase timings on stderr, bit 1 k_solve cycle counts
-
-void set_error(const char* fmt, ...) {
-  char buf[1024];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  g_last_error = buf;
-}
-
-#define CUDA_TRY(expr)                                                                \
-  do {                                                                                \
-    cudaError_t e_ = (expr);                                                          \
-    if (e_ != cudaSuccess) {                                                          \
-      set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
-      return TSCM_ERR_CUDA;                                                           \
-    }                                                                                 \
-  } while (0)
-#define RC_TRY(expr)            \
-  do {                          \
-    const int rc_ = (expr);     \
-    if (rc_) return rc_;        \
-  } while (0)
 
 using Clock = std::chrono::steady_clock;
 double ms_since(Clock::time_point t0) {
@@ -900,31 +881,24 @@ int upload_observations(tscm_solver* s, const double* obs_xy, const std::vector<
   return TSCM_OK;
 }
 
-// One shard on one device.  p->obs_xy may be NULL (uploaded later).
-int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool is_kid, tscm_solver** out) {
+// One shard on the device select_device() made current.  p->obs_xy may be NULL (uploaded later).
+int create_shard(const tscm_problem* p, const tscm_options* o, const internal::SelectedDevice& dev, bool is_kid,
+                 tscm_solver** out) {
   *out = nullptr;
   const auto t0 = Clock::now();
   auto lap = [&](const char* what) {
     if (g_debug & 1) std::fprintf(stderr, "[tscm create] %-28s %8.2f ms\n", what, ms_since(t0));
   };
-  DeviceInfo info;
-  RC_TRY(device_info(device, &info));
-  if (info.major < 10) {
-    set_error("device %d is sm_%d%d; this library is built for sm_100a only", device, info.major, info.minor);
-    return TSCM_ERR_NO_DEVICE;
-  }
-  CUDA_TRY(cudaSetDevice(device));
-  tscm_solver* s = new tscm_solver();
-  s->device = device;
-  s->sm_count = info.sm_count;
-  s->smem_optin = info.smem_optin;
+  std::unique_ptr<tscm_solver, void (*)(tscm_solver*)> owner(new tscm_solver(), free_shard);
+  tscm_solver* s = owner.get();
+  s->device = dev.index;
+  s->sm_count = dev.sm_count;
+  s->smem_optin = dev.smem_optin;
   s->is_kid = is_kid;
   s->use_pdl = (g_debug & 4) == 0;
   s->options = *o;
   fill_lm_options(*o, s->lm);
-#define TRY_S(x) do { const int rc_ = (x); if (rc_) { free_shard(s); return rc_; } } while (0)
-#define CUDA_S(x) do { const cudaError_t e_ = (x); if (e_ != cudaSuccess) { set_error("%s failed: %s (%s:%d)", #x, cudaGetErrorString(e_), __FILE__, __LINE__); free_shard(s); return TSCM_ERR_CUDA; } } while (0)
-  CUDA_S(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
+  CUDA_TRY(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
   const int C = p->num_cameras, F = p->num_frames, K = p->corners_per_board, V = p->num_views;
   s->C = C; s->F = F; s->K = K; s->V = V; s->fixed_camera = p->fixed_camera;
   DeviceProblem& P = s->P;
@@ -953,7 +927,7 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
     set_error("reduced system of %d live parameters (%d cameras) exceeds the limit of %d (16 cameras with one "
               "fixed): the solve needs %zu bytes of shared memory per block, the device allows %zu",
               NL, C, kCovMaxNL, s->solve.smem, s->smem_optin);
-    free_shard(s); return TSCM_ERR_UNSUPPORTED;
+    return TSCM_ERR_UNSUPPORTED;
   }
   std::vector<short> live_cam(NL), live_kk(NL);
   for (int c = 0; c < C; ++c)
@@ -986,7 +960,7 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
       for (int v = 32 * b; v < std::min(V, 32 * b + 32); ++v)
         if (p->view_camera[v] != last) {
           last = p->view_camera[v];
-          if (last < prev_cam) { set_error("internal: slot table"); free_shard(s); return TSCM_ERR_INVALID_ARGUMENT; }
+          if (last < prev_cam) { set_error("internal: slot table"); return TSCM_ERR_INVALID_ARGUMENT; }
           prev_cam = last;
           cam_slot_begin[last + 1]++;
           ++nslot;
@@ -1021,7 +995,7 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   if (s->eval5_smem > s->smem_optin) {
     set_error("problem (%d corners, %d cameras) needs %zu bytes of shared memory per CTA in k_eval5 (limit %zu)", K, C,
               s->eval5_smem, s->smem_optin);
-    free_shard(s); return TSCM_ERR_UNSUPPORTED;
+    return TSCM_ERR_UNSUPPORTED;
   }
   lap("index tables (host)");
 
@@ -1048,7 +1022,7 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   blob.add(&s->schur.tile_bi, tile_bi);
   blob.add(&s->schur.tile_bj, tile_bj);
   const int form = choose_schur_form(s);
-  TRY_S(plan_schur(s, form, A, blob));
+  RC_TRY(plan_schur(s, form, A, blob));
   lap("Schur tables (host)");
 
   // ---- buffers ----------------------------------------------------------------------------
@@ -1111,20 +1085,20 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
   const int cap = std::max(128, std::min(s->options.max_num_iterations, 1 << 16) + 2);
   A.want(&s->d_trace, trace_bytes(cap));
   A.want(&s->d_blob, blob.bytes.size());
-  TRY_S(A.commit(s->stream));
+  RC_TRY(A.commit(s->stream));
   blob.d_base = s->d_blob;
-  TRY_S(blob.upload(s->stream));
+  RC_TRY(blob.upload(s->stream));
   lap("arena + table upload");
   P.obsT = s->d_obsT;
   s->schur.Spart = s->d_Spart; s->schur.rpart = s->d_rpart;
   s->schur.scale_e = s->d_scale_e; s->schur.scale_c = s->d_scale_c;
   wire_trace(s, cap);
-  CUDA_S(cudaMallocHost((void**)&s->h_state, 3 * sizeof(LmState)));
-  CUDA_S(cudaMallocHost((void**)&s->h_err, sizeof(int)));
+  CUDA_TRY(cudaMallocHost((void**)&s->h_state, 3 * sizeof(LmState)));
+  CUDA_TRY(cudaMallocHost((void**)&s->h_err, sizeof(int)));
   *s->h_err = 0;
-  CUDA_S(cudaMallocHost((void**)&s->h_trace, trace_bytes(cap)));
-  CUDA_S(cudaEventCreateWithFlags(&s->poll_ev[0], cudaEventDisableTiming));
-  CUDA_S(cudaEventCreateWithFlags(&s->poll_ev[1], cudaEventDisableTiming));
+  CUDA_TRY(cudaMallocHost((void**)&s->h_trace, trace_bytes(cap)));
+  CUDA_TRY(cudaEventCreateWithFlags(&s->poll_ev[0], cudaEventDisableTiming));
+  CUDA_TRY(cudaEventCreateWithFlags(&s->poll_ev[1], cudaEventDisableTiming));
   {
     // mailbox of the peer-memory exchange (tiny; its own allocation so that its IPC handle can
     // be exported right after creation)
@@ -1133,29 +1107,27 @@ int create_shard(const tscm_problem* p, const tscm_options* o, int device, bool 
     s->p2p.nctaA = (nwords + 31) / 32;
     s->p2p.nB = (C * kCamRec + kCommExtra + 1 + 31) / 32 * 32;
     const size_t words = p2p_mailbox_words(s->p2p.nA, s->p2p.nctaA, s->p2p.nB);
-    CUDA_S(cudaMalloc((void**)&s->d_mailbox, words * sizeof(double)));
-    CUDA_S(cudaMemsetAsync(s->d_mailbox, 0, words * sizeof(double), s->stream));
+    CUDA_TRY(cudaMalloc((void**)&s->d_mailbox, words * sizeof(double)));
+    CUDA_TRY(cudaMemsetAsync(s->d_mailbox, 0, words * sizeof(double), s->stream));
     s->p2p.seq = s->d_p2p_seq; s->p2p.ticket = s->d_p2p_ticket; s->p2p.err = s->d_p2p_err;
     s->p2p.timeout_ns = 10ull * 1000000000ull;
   }
-  TRY_S(wire_schur(s, form));
+  RC_TRY(wire_schur(s, form));
   if (s->use_cluster) {
-    TRY_S(ensure_cluster(s));
+    RC_TRY(ensure_cluster(s));
   } else {
-    TRY_S(set_smem_attr((const void*)k_solve<1, 4>, s->solve.smem));
-    TRY_S(set_smem_attr((const void*)k_solve<4, 7>, s->solve.smem));
+    RC_TRY(set_smem_attr((const void*)k_solve<1, 4>, s->solve.smem));
+    RC_TRY(set_smem_attr((const void*)k_solve<4, 7>, s->solve.smem));
   }
-  TRY_S(set_smem_attr((const void*)k_eval5, s->eval5_smem));
-  TRY_S(set_smem_attr((const void*)k_view_blocks, vb_smem_bytes()));
+  RC_TRY(set_smem_attr((const void*)k_eval5, s->eval5_smem));
+  RC_TRY(set_smem_attr((const void*)k_view_blocks, vb_smem_bytes()));
   lap("kernel attributes");
   if (p->obs_xy) {
-    TRY_S(upload_observations(s, p->obs_xy, nullptr));
-    CUDA_S(cudaStreamSynchronize(s->stream));
+    RC_TRY(upload_observations(s, p->obs_xy, nullptr));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
     lap("observations H2D + transpose");
   }
-#undef TRY_S
-#undef CUDA_S
-  *out = s;
+  *out = owner.release();
   return TSCM_OK;
 }
 
@@ -1211,15 +1183,17 @@ void destroy_solver(tscm_solver* s) {
   free_shard(s);
 }
 
-int create_group(const tscm_problem* p, const tscm_options* o, int device, int n, tscm_solver** out) {
-  int ndev = 0;
-  CUDA_TRY(cudaGetDeviceCount(&ndev));
-  if (device + n > ndev) {
-    set_error("num_gpus = %d from device %d, but only %d device(s) are visible", n, device, ndev);
+// `dev`: select_device() of the first device of the group
+int create_group(const tscm_problem* p, const tscm_options* o, const internal::SelectedDevice& dev, int n,
+                 tscm_solver** out) {
+  const int device = dev.index;
+  if (device + n > dev.visible) {
+    set_error("num_gpus = %d from device %d, but only %d device(s) are visible", n, device, dev.visible);
     return TSCM_ERR_NO_DEVICE;
   }
   if (p->num_frames < n) { set_error("%d frames cannot be sharded over %d GPUs", p->num_frames, n); return TSCM_ERR_INVALID_ARGUMENT; }
-  tscm_solver* g = new tscm_solver();
+  std::unique_ptr<tscm_solver, void (*)(tscm_solver*)> owner(new tscm_solver(), destroy_solver);
+  tscm_solver* g = owner.get();
   g->device = device;
   g->options = *o;
   g->C = p->num_cameras; g->F = p->num_frames; g->K = p->corners_per_board; g->V = p->num_views;
@@ -1239,9 +1213,10 @@ int create_group(const tscm_problem* p, const tscm_options* o, int device, int n
     q.view_camera = sp.vcam[r].data();
     q.view_frame = sp.vfrm[r].data();
     q.obs_xy = nullptr;
+    internal::SelectedDevice kd;
+    RC_TRY(internal::select_device(device + r, "the calibration solve", &kd));
     tscm_solver* k = nullptr;
-    const int rc = create_shard(&q, o, device + r, true, &k);
-    if (rc) { destroy_solver(g); return rc; }
+    RC_TRY(create_shard(&q, o, kd, true, &k));
     k->obs_count = g->obs_count;      // global counts: the read-out divides global sums
     g->kids.push_back(k);
   }
@@ -1252,10 +1227,10 @@ int create_group(const tscm_problem* p, const tscm_options* o, int device, int n
       if (i == j) continue;
       int can = 0;
       cudaDeviceCanAccessPeer(&can, device + i, device + j);
-      if (!can) { set_error("device %d cannot access device %d: num_gpus needs peer access", device + i, device + j); destroy_solver(g); return TSCM_ERR_UNSUPPORTED; }
+      if (!can) { set_error("device %d cannot access device %d: num_gpus needs peer access", device + i, device + j); return TSCM_ERR_UNSUPPORTED; }
       const cudaError_t e = cudaDeviceEnablePeerAccess(device + j, 0);
       if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
-      else if (e != cudaSuccess) { set_error("cudaDeviceEnablePeerAccess(%d -> %d): %s", device + i, device + j, cudaGetErrorString(e)); destroy_solver(g); return TSCM_ERR_CUDA; }
+      else if (e != cudaSuccess) { set_error("cudaDeviceEnablePeerAccess(%d -> %d): %s", device + i, device + j, cudaGetErrorString(e)); return TSCM_ERR_CUDA; }
     }
   }
   for (int i = 0; i < n; ++i) {
@@ -1272,23 +1247,12 @@ int create_group(const tscm_problem* p, const tscm_options* o, int device, int n
     k->graph_dirty = true;
   }
   if (p->obs_xy) {
-    for (int i = 0; i < n; ++i) {
-      const int rc = upload_observations(g->kids[i], p->obs_xy, &g->kid_seg[i]);
-      if (rc) { destroy_solver(g); return rc; }
-    }
+    for (int i = 0; i < n; ++i) RC_TRY(upload_observations(g->kids[i], p->obs_xy, &g->kid_seg[i]));
     for (tscm_solver* k : g->kids) { cudaSetDevice(k->device); cudaStreamSynchronize(k->stream); }
   }
-  *out = g;
+  *out = owner.release();
   return TSCM_OK;
 }
-
-// The library switches devices (shards of a group, an explicit `device` argument); the caller's
-// current device is restored on the way out of every entry point.
-struct DeviceGuard {
-  int prev = -1;
-  DeviceGuard() { if (cudaGetDevice(&prev) != cudaSuccess) { prev = -1; cudaGetLastError(); } }
-  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
 
 // every shard (or the solver itself)
 template <typename Fn>
@@ -1308,6 +1272,38 @@ int sync_shards(tscm_solver* s) {
   });
 }
 tscm_solver* lead(tscm_solver* s) { return s->kids.empty() ? s : s->kids[0]; }
+
+// The evaluation records of the read-outs: every shard evaluates its current point, under the
+// plain (loss-free) residuals with the sum of sqrt(s) if `want_err`, or under the configured loss
+// (plain = false: the records a later run() starts from), and the records are summed over the
+// shards or ranks.  Waits for every shard.
+int evaluate_shards(tscm_solver* s, bool plain, bool want_err) {
+  RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
+    CUDA_TRY(cudaSetDevice(k->device));
+    const int cur = k->x_in_set1 ? 1 : 0;
+    const LmOptions saved = k->lm;
+    if (plain) k->lm.loss_type = 0;
+    k->want_err = want_err ? 1 : 0;
+    launch_evaluation(k, 2 + cur, 1);
+    const int rc = launch_eval_allreduce(k, 2 + cur);
+    k->lm = saved;
+    k->want_err = 0;
+    return rc;
+  }));
+  return sync_shards(s);
+}
+
+// Sums a host record of C * kCamRec + kCommExtra doubles over the ranks of a multi-process solve,
+// in place, through the exchange of the evaluation record (which it overwrites).
+int allreduce_record(tscm_solver* L, std::vector<double>& rec) {
+  const int cur = L->x_in_set1 ? 1 : 0;
+  CUDA_TRY(cudaSetDevice(L->device));
+  CUDA_TRY(cudaMemcpyAsync(L->ps[cur].comm, rec.data(), rec.size() * sizeof(double), cudaMemcpyHostToDevice, L->stream));
+  RC_TRY(launch_eval_allreduce(L, 2 + cur));
+  CUDA_TRY(cudaStreamSynchronize(L->stream));
+  CUDA_TRY(cudaMemcpy(rec.data(), L->ps[cur].comm, rec.size() * sizeof(double), cudaMemcpyDeviceToHost));
+  return TSCM_OK;
+}
 
 // ---------------------------------------------------------------------------
 // solver cache of tscm_solve()
@@ -1375,6 +1371,43 @@ void cache_checkin(tscm_solver* s, int device, int ngpu, bool keep) {
   }
 }
 
+// The solver of a one-shot call (tscm_solve, tscm_compute_covariance) on a validated problem:
+// validates the options, selects the device, takes the cached solver of this structure (with the
+// options set) or creates one, and uploads the observations.  Hand it back with cache_checkin().
+struct Checkout {
+  tscm_solver* s = nullptr;
+  int device = 0, ngpu = 1;
+  bool hit = false;
+};
+int checkout_solver(const tscm_problem* problem, const tscm_options* options, int device, const char* what,
+                    Checkout* c) {
+  tscm_options defaults;
+  tscm_options_init(&defaults);
+  if (!options) options = &defaults;
+  RC_TRY(validate_options(options));
+  RC_TRY(validate_large_rig(problem, options));
+  internal::SelectedDevice dev;
+  RC_TRY(internal::select_device(device, what, &dev));
+  c->device = dev.index;
+  c->ngpu = std::max(1, options->num_gpus);
+  c->s = cache_checkout(problem, c->device, c->ngpu, options->allow_large_rigs);
+  c->hit = c->s != nullptr;
+  int rc = TSCM_OK;
+  if (c->hit) {
+    rc = tscm_solver_set_options(c->s, options);
+  } else {
+    tscm_problem q = *problem;
+    q.obs_xy = nullptr;                        // uploaded below, without a sync of its own
+    rc = tscm_solver_create(&q, options, c->device, &c->s);
+  }
+  if (!rc) rc = upload_all_observations(c->s, problem->obs_xy);
+  if (rc && c->s) {
+    destroy_solver(c->s);
+    c->s = nullptr;
+  }
+  return rc;
+}
+
 // ---------------------------------------------------------------------------
 // covariance (tscm_covariance.cuh)
 // ---------------------------------------------------------------------------
@@ -1433,25 +1466,30 @@ void set_error(const char* fmt, ...) {
   va_start(ap, fmt);
   vsnprintf(buf, sizeof(buf), fmt, ap);
   va_end(ap);
-  ::set_error("%s", buf);
+  g_last_error = buf;
 }
-int select_device(int device, const char* what, int* sm_count) {
+int select_device(int device, const char* what, SelectedDevice* out) {
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     cudaGetLastError();
-    ::set_error("no CUDA device: %s has no CPU fallback", what);
+    set_error("no CUDA device: %s has no CPU fallback", what);
     return TSCM_ERR_NO_DEVICE;
   }
-  if (device >= 0) CUDA_TRY(cudaSetDevice(device));
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
+  if (device < 0) CUDA_TRY(cudaGetDevice(&device));
+  if (device >= ndev) { set_error("device %d does not exist (%d visible)", device, ndev); return TSCM_ERR_NO_DEVICE; }
   DeviceInfo prop;
-  RC_TRY(device_info(dev, &prop));
+  RC_TRY(device_info(device, &prop));
   if (prop.major < 10) {
-    ::set_error("device %d is sm_%d%d; this library is built for sm_100a only", dev, prop.major, prop.minor);
+    set_error("device %d is sm_%d%d; this library is built for sm_100a only", device, prop.major, prop.minor);
     return TSCM_ERR_NO_DEVICE;
   }
-  if (sm_count) *sm_count = prop.sm_count;
+  CUDA_TRY(cudaSetDevice(device));
+  if (out) {
+    out->index = device;
+    out->visible = ndev;
+    out->sm_count = prop.sm_count;
+    out->smem_optin = prop.smem_optin;
+  }
   return TSCM_OK;
 }
 DeviceScope::DeviceScope() { if (cudaGetDevice(&prev) != cudaSuccess) { prev = -1; cudaGetLastError(); } }
@@ -1540,7 +1578,7 @@ int tscm_solver_set_options(tscm_solver* s, const tscm_options* o) {
 }
 
 int tscm_solver_create(const tscm_problem* p, const tscm_options* o, int device, tscm_solver** out) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!out) { set_error("out is NULL"); return TSCM_ERR_INVALID_ARGUMENT; }
   *out = nullptr;
   const auto t0 = Clock::now();
@@ -1550,27 +1588,21 @@ int tscm_solver_create(const tscm_problem* p, const tscm_options* o, int device,
   if (!o) o = &defaults;
   RC_TRY(validate_options(o));
   RC_TRY(validate_large_rig(p, o));
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    set_error("no CUDA device: the calibration solve has no CPU fallback");
-    return TSCM_ERR_NO_DEVICE;
-  }
-  if (device < 0) CUDA_TRY(cudaGetDevice(&device));
-  if (device >= ndev) { set_error("device %d does not exist (%d visible)", device, ndev); return TSCM_ERR_NO_DEVICE; }
+  internal::SelectedDevice dev;
+  RC_TRY(internal::select_device(device, "the calibration solve", &dev));
   if (g_debug & 1) std::fprintf(stderr, "[tscm create] %-28s %8.2f ms\n", "validate", ms_since(t0));
   const int n = std::max(1, o->num_gpus);
-  if (n > 1) return create_group(p, o, device, n, out);
-  return create_shard(p, o, device, false, out);
+  if (n > 1) return create_group(p, o, dev, n, out);
+  return create_shard(p, o, dev, false, out);
 }
 
 void tscm_solver_destroy(tscm_solver* s) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   destroy_solver(s);
 }
 
 int tscm_solver_set_observations(tscm_solver* s, const double* obs_xy) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || !obs_xy) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   RC_TRY(upload_all_observations(s, obs_xy));
   return sync_shards(s);     // the caller may reuse obs_xy
@@ -1578,7 +1610,7 @@ int tscm_solver_set_observations(tscm_solver* s, const double* obs_xy) {
 
 int tscm_solver_set_parameters(tscm_solver* s, const double* intr, const double* cam_rt,
                                const double* board_rt) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || !intr || !cam_rt || !board_rt) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   RC_TRY(for_shards(s, [&](tscm_solver* k, int i) -> int {
     CUDA_TRY(cudaSetDevice(k->device));
@@ -1598,7 +1630,7 @@ int tscm_solver_set_parameters(tscm_solver* s, const double* intr, const double*
 }
 
 int tscm_solver_get_parameters(tscm_solver* s, double* intr, double* cam_rt, double* board_rt) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   RC_TRY(for_shards(s, [&](tscm_solver* k, int i) -> int {
     CUDA_TRY(cudaSetDevice(k->device));
@@ -1613,7 +1645,7 @@ int tscm_solver_get_parameters(tscm_solver* s, double* intr, double* cam_rt, dou
 }
 
 int tscm_solver_run(tscm_solver* s, tscm_summary* summary) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   const int max_it = s->options.max_num_iterations;
   // ---- prepare every shard (no exchange kernels yet) -----------------------------------------
@@ -1709,14 +1741,14 @@ int tscm_solver_run(tscm_solver* s, tscm_summary* summary) {
 }
 
 void tscm_cache_configure(int32_t max_solvers) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   std::lock_guard<std::mutex> lock(g_cache_mu);
   g_cache_max = std::max(0, (int)max_solvers);
   while ((int)g_cache.size() > g_cache_max) cache_evict_oldest_locked();
   if (g_cache_max == 0 && g_host_block && !g_host_busy) { cudaFreeHost(g_host_block); g_host_block = nullptr; g_host_bytes = 0; }
 }
 void tscm_cache_release(void) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   std::lock_guard<std::mutex> lock(g_cache_mu);
   for (CacheEntry& e : g_cache) destroy_solver(e.solver);
   g_cache.clear();
@@ -1725,48 +1757,27 @@ void tscm_cache_release(void) {
 
 int tscm_solve(const tscm_problem* problem, const tscm_options* options, double* intrinsics,
                double* cam_rt, double* board_rt, tscm_summary* summary, int device) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   const auto t0 = Clock::now();
   RC_TRY(validate_problem(problem, true));
   if (!intrinsics || !cam_rt || !board_rt) { set_error("NULL parameter arrays"); return TSCM_ERR_INVALID_ARGUMENT; }
-  tscm_options defaults;
-  tscm_options_init(&defaults);
-  if (!options) options = &defaults;
-  RC_TRY(validate_options(options));
-  RC_TRY(validate_large_rig(problem, options));
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    set_error("no CUDA device: the calibration solve has no CPU fallback");
-    return TSCM_ERR_NO_DEVICE;
-  }
-  if (device < 0) CUDA_TRY(cudaGetDevice(&device));
-  const int ngpu = std::max(1, options->num_gpus);
   // ---- solver: cached for this structure, or new ---------------------------------------------
-  tscm_solver* s = cache_checkout(problem, device, ngpu, options->allow_large_rigs);
-  const bool hit = s != nullptr;
   const double ms_lookup = ms_since(t0);
-  int rc = TSCM_OK;
-  if (hit) {
-    rc = tscm_solver_set_options(s, options);
-  } else {
-    tscm_problem q = *problem;
-    q.obs_xy = nullptr;                        // uploaded below, without a sync of its own
-    rc = tscm_solver_create(&q, options, device, &s);
-  }
-  if (!rc) rc = upload_all_observations(s, problem->obs_xy);
+  Checkout c;
+  RC_TRY(checkout_solver(problem, options, device, "the calibration solve", &c));
+  tscm_solver* s = c.s;
   const double ms_create = ms_since(t0);
   // the parameters ride behind the observations on the same streams (one sync for both)
-  if (!rc) rc = tscm_solver_set_parameters(s, intrinsics, cam_rt, board_rt);
+  int rc = tscm_solver_set_parameters(s, intrinsics, cam_rt, board_rt);
   const double ms_set = ms_since(t0);
   if (!rc) rc = tscm_solver_run(s, summary);
   const double ms_run = ms_since(t0);
   if (!rc) rc = tscm_solver_get_parameters(s, intrinsics, cam_rt, board_rt);
   const double ms_get = ms_since(t0);
-  if (s) cache_checkin(s, device, ngpu, rc == TSCM_OK);
+  cache_checkin(s, c.device, c.ngpu, rc == TSCM_OK);
   if (g_debug & 1)
     std::fprintf(stderr, "[tscm_solve] %s: lookup %.2f  create/upload %.2f  set %.2f  run %.2f  get %.2f  total %.2f ms\n",
-                 hit ? "cached solver" : "new solver", ms_lookup, ms_create - ms_lookup, ms_set - ms_create,
+                 c.hit ? "cached solver" : "new solver", ms_lookup, ms_create - ms_lookup, ms_set - ms_create,
                  ms_run - ms_set, ms_get - ms_run, ms_since(t0));
   return rc;
 }
@@ -1797,7 +1808,7 @@ static int no_large_shards(const tscm_solver* s) {
 }
 
 int tscm_solver_attach_comm(tscm_solver* s, int rank, int num_ranks, const void* unique_id_128) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || !unique_id_128 || rank < 0 || rank >= num_ranks) { set_error("bad comm arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_attach_comm");
   RC_TRY(no_large_shards(s));
@@ -1814,7 +1825,7 @@ int tscm_solver_attach_comm(tscm_solver* s, int rank, int num_ranks, const void*
 }
 
 int tscm_solver_p2p_export(tscm_solver* s, void* handle_64) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || !handle_64) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_p2p_export");
   static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
@@ -1827,7 +1838,7 @@ int tscm_solver_p2p_export(tscm_solver* s, void* handle_64) {
 }
 
 int tscm_solver_p2p_attach(tscm_solver* s, int rank, int num_ranks, const void* handles) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || !handles || rank < 0 || rank >= num_ranks) { set_error("bad p2p arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_p2p_attach");
   RC_TRY(no_large_shards(s));
@@ -1863,7 +1874,7 @@ int tscm_solver_set_exchange_timeout(tscm_solver* s, double seconds) {
 }
 
 int tscm_solver_set_schur_form(tscm_solver* s, int form) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   return for_shards(s, [&](tscm_solver* k, int) -> int {
     CUDA_TRY(cudaSetDevice(k->device));
@@ -1884,7 +1895,7 @@ int tscm_solver_set_schur_form(tscm_solver* s, int form) {
 }
 
 int tscm_solver_set_reduced_solve(tscm_solver* s, int form) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || form < 0 || form > 2) { set_error("bad arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   return for_shards(s, [&](tscm_solver* k, int) -> int {
     CUDA_TRY(cudaSetDevice(k->device));
@@ -1909,15 +1920,16 @@ int tscm_solver_set_reduced_solve(tscm_solver* s, int form) {
 }
 
 int tscm_solver_eval_jacobian(tscm_solver* s, double* residuals, double* jacobian, double* cost) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_eval_jacobian");
   CUDA_TRY(cudaSetDevice(s->device));
   const int cur = s->x_in_set1 ? 1 : 0;
   const size_t N = (size_t)s->V * s->K;
+  internal::Scratch scratch;
   double *d_r = nullptr, *d_J = nullptr;
-  if (residuals) CUDA_TRY(cudaMalloc((void**)&d_r, N * 2 * sizeof(double)));
-  if (jacobian) CUDA_TRY(cudaMalloc((void**)&d_J, N * 42 * sizeof(double)));
+  if (residuals) CUDA_TRY(scratch.alloc(&d_r, N * 2));
+  if (jacobian) CUDA_TRY(scratch.alloc(&d_J, N * 42));
   k_prep_cams<<<(s->C + 31) / 32, 32, 0, s->stream>>>(s->P, s->ps[0], s->ps[1], s->d_state, 2 + cur);
   k_eval_rows<<<(unsigned)((N + 127) / 128), 128, 0, s->stream>>>(s->P, s->ps[cur], s->lm, d_r, d_J);
   s->launches += 2;
@@ -1927,8 +1939,8 @@ int tscm_solver_eval_jacobian(tscm_solver* s, double* residuals, double* jacobia
   }
   CUDA_TRY(cudaStreamSynchronize(s->stream));
   CUDA_TRY(cudaGetLastError());
-  if (residuals) { CUDA_TRY(cudaMemcpy(residuals, d_r, N * 2 * sizeof(double), cudaMemcpyDeviceToHost)); cudaFree(d_r); }
-  if (jacobian) { CUDA_TRY(cudaMemcpy(jacobian, d_J, N * 42 * sizeof(double), cudaMemcpyDeviceToHost)); cudaFree(d_J); }
+  if (residuals) CUDA_TRY(cudaMemcpy(residuals, d_r, N * 2 * sizeof(double), cudaMemcpyDeviceToHost));
+  if (jacobian) CUDA_TRY(cudaMemcpy(jacobian, d_J, N * 42 * sizeof(double), cudaMemcpyDeviceToHost));
   if (cost) {
     std::vector<double> comm((size_t)s->C * kCamRec);
     CUDA_TRY(cudaMemcpy(comm.data(), s->ps[cur].comm, comm.size() * sizeof(double), cudaMemcpyDeviceToHost));
@@ -1945,7 +1957,7 @@ int tscm_solver_reduced_size(const tscm_solver* s) {
 }
 
 int tscm_solver_reduced_system(tscm_solver* s, double radius, double* lhs, double* rhs) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || !(radius > 0.0)) { set_error("bad arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   NO_GROUP(s, "tscm_solver_reduced_system");
   CUDA_TRY(cudaSetDevice(s->device));
@@ -1969,25 +1981,11 @@ int tscm_solver_reduced_system(tscm_solver* s, double radius, double* lhs, doubl
 // sharded solve (ranks or a num_gpus group) the sums are global, and so must the counts be: a
 // group knows them; the ranks of a multi-process solve exchange them like an evaluation record.
 int tscm_solver_reprojection_error(tscm_solver* s, double* per_camera, double* overall, double* rms) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   const int C = s->C;
   // Read-out uses the plain (loss-free) residuals, like multi_calib.cpp:235-283.
-  auto evaluate = [&](bool plain) -> int {
-    RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
-      CUDA_TRY(cudaSetDevice(k->device));
-      const int cur = k->x_in_set1 ? 1 : 0;
-      const LmOptions saved = k->lm;
-      if (plain) { k->lm.loss_type = 0; k->want_err = 1; }
-      launch_evaluation(k, 2 + cur, 1);
-      const int rc = launch_eval_allreduce(k, 2 + cur);
-      k->lm = saved;
-      k->want_err = 0;
-      return rc;
-    }));
-    return sync_shards(s);
-  };
-  RC_TRY(evaluate(true));
+  RC_TRY(evaluate_shards(s, /*plain=*/true, /*want_err=*/true));
   tscm_solver* L = lead(s);
   const int cur = L->x_in_set1 ? 1 : 0;
   CUDA_TRY(cudaSetDevice(L->device));
@@ -2000,10 +1998,7 @@ int tscm_solver_reprojection_error(tscm_solver* s, double* per_camera, double* o
     // exchange the local counts through the record's err slot
     std::vector<double> rec((size_t)C * kCamRec + kCommExtra, 0.0);
     for (int m = 0; m < C; ++m) rec[(size_t)m * kCamRec + kCamErr] = L->obs_count[m];
-    CUDA_TRY(cudaMemcpyAsync(L->ps[cur].comm, rec.data(), rec.size() * sizeof(double), cudaMemcpyHostToDevice, L->stream));
-    RC_TRY(launch_eval_allreduce(L, 2 + cur));
-    CUDA_TRY(cudaStreamSynchronize(L->stream));
-    CUDA_TRY(cudaMemcpy(rec.data(), L->ps[cur].comm, rec.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    RC_TRY(allreduce_record(L, rec));
     for (int m = 0; m < C; ++m) count[m] = rec[(size_t)m * kCamRec + kCamErr];
   }
   double sum = 0.0, cost = 0.0, total = 0.0;
@@ -2017,7 +2012,7 @@ int tscm_solver_reprojection_error(tscm_solver* s, double* per_camera, double* o
   if (overall) *overall = total > 0 ? sum / total : 0.0;
   if (rms) *rms = total > 0 ? std::sqrt(2.0 * cost / total) : 0.0;
   // restore the records of the configured loss for a subsequent run()
-  if (L->lm.loss_type || multi_process) RC_TRY(evaluate(false));
+  if (L->lm.loss_type || multi_process) RC_TRY(evaluate_shards(s, /*plain=*/false, /*want_err=*/false));
   return TSCM_OK;
 }
 
@@ -2025,25 +2020,18 @@ int tscm_solver_reprojection_error(tscm_solver* s, double* per_camera, double* o
 // Collective on a sharded solve, like run(): every shard assembles the undamped system over the
 // usual exchange and inverts S~ redundantly; each shard computes the blocks of its own frames.
 int tscm_solver_covariance(tscm_solver* s, tscm_covariance* out) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || !out) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
   const int C = s->C;
   tscm_solver* L = lead(s);
   const int NL = L->P.NL;
   const bool multi_process = s->kids.empty() && s->num_ranks > 1;
-  // sum |r|^2 of the plain (loss-free) residuals
   RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
     CUDA_TRY(cudaSetDevice(k->device));
-    RC_TRY(ensure_cov_buffers(k));
-    const int cur = k->x_in_set1 ? 1 : 0;
-    const LmOptions saved = k->lm;
-    k->lm.loss_type = 0;
-    launch_evaluation(k, 2 + cur, 1);
-    const int rc = launch_eval_allreduce(k, 2 + cur);
-    k->lm = saved;
-    return rc;
+    return ensure_cov_buffers(k);
   }));
-  RC_TRY(sync_shards(s));
+  // sum |r|^2 of the plain (loss-free) residuals
+  RC_TRY(evaluate_shards(s, /*plain=*/true, /*want_err=*/false));
   const int cur = L->x_in_set1 ? 1 : 0;
   CUDA_TRY(cudaSetDevice(L->device));
   CUDA_TRY(cudaGetLastError());
@@ -2080,22 +2068,16 @@ int tscm_solver_covariance(tscm_solver* s, tscm_covariance* out) {
   std::vector<double> count = L->obs_count;
   double frames = s->F;
   if (multi_process) {
-    CUDA_TRY(cudaSetDevice(L->device));
     std::fill(rec.begin(), rec.end(), 0.0);
     for (int m = 0; m < C; ++m) rec[(size_t)m * kCamRec + kCamErr] = L->obs_count[m];
     rec[kCamCost] = L->F;
     rec[(size_t)C * kCamRec] = (flag & 2) ? 1.0 : 0.0;
-    CUDA_TRY(cudaMemcpyAsync(L->ps[cur].comm, rec.data(), rec.size() * sizeof(double), cudaMemcpyHostToDevice, L->stream));
-    RC_TRY(launch_eval_allreduce(L, 2 + cur));
-    CUDA_TRY(cudaStreamSynchronize(L->stream));
-    CUDA_TRY(cudaMemcpy(rec.data(), L->ps[cur].comm, rec.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    RC_TRY(allreduce_record(L, rec));
     for (int m = 0; m < C; ++m) count[m] = rec[(size_t)m * kCamRec + kCamErr];
     frames = rec[kCamCost];
     if (rec[(size_t)C * kCamRec] > 0.0) flag |= 2;
     // restore the records of the configured loss
-    launch_evaluation(L, 2 + cur, 1);
-    RC_TRY(launch_eval_allreduce(L, 2 + cur));
-    CUDA_TRY(cudaStreamSynchronize(L->stream));
+    RC_TRY(evaluate_shards(s, /*plain=*/false, /*want_err=*/false));
     CUDA_TRY(cudaGetLastError());
   }
   if (flag) {
@@ -2132,41 +2114,20 @@ int tscm_solver_covariance(tscm_solver* s, tscm_covariance* out) {
 
 int tscm_compute_covariance(const tscm_problem* problem, const tscm_options* options, const double* intrinsics,
                     const double* cam_rt, const double* board_rt, tscm_covariance* cov, int device) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   RC_TRY(validate_problem(problem, true));
   if (!intrinsics || !cam_rt || !board_rt || !cov) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
-  tscm_options defaults;
-  tscm_options_init(&defaults);
-  if (!options) options = &defaults;
-  RC_TRY(validate_options(options));
-  RC_TRY(validate_large_rig(problem, options));
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    set_error("no CUDA device: the covariance has no CPU fallback");
-    return TSCM_ERR_NO_DEVICE;
-  }
-  if (device < 0) CUDA_TRY(cudaGetDevice(&device));
-  const int ngpu = std::max(1, options->num_gpus);
   // the solver cache of tscm_solve(): after a solve of this structure only data is uploaded
-  tscm_solver* s = cache_checkout(problem, device, ngpu, options->allow_large_rigs);
-  int rc = TSCM_OK;
-  if (s) {
-    rc = tscm_solver_set_options(s, options);
-  } else {
-    tscm_problem q = *problem;
-    q.obs_xy = nullptr;
-    rc = tscm_solver_create(&q, options, device, &s);
-  }
-  if (!rc) rc = upload_all_observations(s, problem->obs_xy);
-  if (!rc) rc = tscm_solver_set_parameters(s, intrinsics, cam_rt, board_rt);
-  if (!rc) rc = tscm_solver_covariance(s, cov);
-  if (s) cache_checkin(s, device, ngpu, rc == TSCM_OK || rc == TSCM_ERR_RANK_DEFICIENT);
+  Checkout c;
+  RC_TRY(checkout_solver(problem, options, device, "the covariance", &c));
+  int rc = tscm_solver_set_parameters(c.s, intrinsics, cam_rt, board_rt);
+  if (!rc) rc = tscm_solver_covariance(c.s, cov);
+  cache_checkin(c.s, c.device, c.ngpu, rc == TSCM_OK || rc == TSCM_ERR_RANK_DEFICIENT);
   return rc;
 }
 
 int tscm_solver_time_stage(tscm_solver* s, int stage, int repeats, double* ms_per_launch) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!s || repeats <= 0 || !ms_per_launch) { set_error("bad arguments"); return TSCM_ERR_INVALID_ARGUMENT; }
   if (stage != 4) NO_GROUP(s, "tscm_solver_time_stage (stages other than 4)");
   RC_TRY(for_shards(s, [&](tscm_solver* k, int) -> int {
@@ -2176,9 +2137,8 @@ int tscm_solver_time_stage(tscm_solver* s, int stage, int repeats, double* ms_pe
   }));
   tscm_solver* L = lead(s);
   CUDA_TRY(cudaSetDevice(L->device));
-  cudaEvent_t e0, e1;
-  CUDA_TRY(cudaEventCreate(&e0));
-  CUDA_TRY(cudaEventCreate(&e1));
+  internal::Scratch timer;
+  CUDA_TRY(timer.create_events());
   if (stage != 4) {
     // make the device state valid and not `done`
     LmOptions saved = s->lm;
@@ -2188,7 +2148,7 @@ int tscm_solver_time_stage(tscm_solver* s, int stage, int repeats, double* ms_pe
     if (!rc) { launch_solve(s); launch_backsub(s); launch_evaluation(s, 3, 0); }
     if (rc) { s->lm = saved; return rc; }
     CUDA_TRY(cudaStreamSynchronize(s->stream));
-    CUDA_TRY(cudaEventRecord(e0, s->stream));
+    CUDA_TRY(cudaEventRecord(timer.e0, s->stream));
     for (int r = 0; r < repeats; ++r) {
       switch (stage) {
         case 0: launch_eval_kernel(s, 3); break;
@@ -2201,7 +2161,7 @@ int tscm_solver_time_stage(tscm_solver* s, int stage, int repeats, double* ms_pe
         default: s->lm = saved; set_error("unknown stage %d", stage); return TSCM_ERR_INVALID_ARGUMENT;
       }
     }
-    CUDA_TRY(cudaEventRecord(e1, s->stream));
+    CUDA_TRY(cudaEventRecord(timer.e1, s->stream));
     s->lm = saved;
   } else {
     // whole LM iterations: iteration zero, then replay the graph.  The options
@@ -2213,7 +2173,7 @@ int tscm_solver_time_stage(tscm_solver* s, int stage, int repeats, double* ms_pe
     }));
     RC_TRY(sync_shards(s));
     CUDA_TRY(cudaSetDevice(L->device));
-    CUDA_TRY(cudaEventRecord(e0, L->stream));
+    CUDA_TRY(cudaEventRecord(timer.e0, L->stream));
     const bool group = !s->kids.empty();
     int left = repeats;
     while (left > 0) {
@@ -2227,16 +2187,14 @@ int tscm_solver_time_stage(tscm_solver* s, int stage, int repeats, double* ms_pe
       left -= n;
     }
     CUDA_TRY(cudaSetDevice(L->device));
-    CUDA_TRY(cudaEventRecord(e1, L->stream));
+    CUDA_TRY(cudaEventRecord(timer.e1, L->stream));
   }
-  CUDA_TRY(cudaEventSynchronize(e1));
+  double ms = 0.0;
+  CUDA_TRY(timer.add_ms(&ms));
   RC_TRY(sync_shards(s));
   CUDA_TRY(cudaSetDevice(L->device));
   CUDA_TRY(cudaGetLastError());
-  float ms = 0.f;
-  CUDA_TRY(cudaEventElapsedTime(&ms, e0, e1));
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  *ms_per_launch = (double)ms / repeats;
+  *ms_per_launch = ms / repeats;
   // where x ended up (the timed stages evaluate set 1 explicitly and never flip `cur`)
   RC_TRY(fetch_state(L));
   const bool in1 = (L->h_state->cur & 1) != 0;
@@ -2260,354 +2218,26 @@ int64_t tscm_solver_launch_count(const tscm_solver* s) {
   return n;
 }
 
-// Remap tables (SURVEY 8f #4): TS.cpp:284-330, rectify.cpp:86-199 as one batched kernel.
-int tscm_remap_tables(const tscm_remap_job* jobs, int32_t num_jobs, int32_t map_width,
-                      int32_t map_height, float* mapx, float* mapy, int device, double* kernel_ms) {
-  DeviceGuard device_guard_;
-  if (!jobs || !mapx || !mapy || num_jobs <= 0 || map_width <= 0 || map_height <= 0) {
-    set_error("bad remap arguments"); return TSCM_ERR_INVALID_ARGUMENT;
-  }
-  if (num_jobs > kRemapMaxJobs) {
-    set_error("%d remap jobs exceed the per-call limit of %d", num_jobs, kRemapMaxJobs);
-    return TSCM_ERR_INVALID_ARGUMENT;
-  }
-  std::vector<RemapBatch> hb(1);
-  RemapBatch& B = hb[0];
-  std::memset(&B, 0, sizeof(B));
-  int64_t total = 0;
-  for (int k = 0; k < num_jobs; ++k) {
-    const tscm_remap_job& j = jobs[k];
-    if (j.width <= 0 || j.height <= 0 || j.row0 < 0 || j.col0 < 0 ||
-        (int64_t)j.row0 + j.height > map_height || (int64_t)j.col0 + j.width > map_width) {
-      set_error("remap job %d: block %dx%d at (%d,%d) does not fit the %dx%d maps", k, j.width, j.height,
-                j.col0, j.row0, map_width, map_height);
-      return TSCM_ERR_INVALID_ARGUMENT;
-    }
-    if (j.ray_fx == 0.0 || j.ray_fy == 0.0) { set_error("remap job %d: zero ray focal length", k); return TSCM_ERR_INVALID_ARGUMENT; }
-    RemapJobDev& d = B.job[k];
-    std::memcpy(d.intr, j.intrinsics, sizeof(d.intr));
-    std::memcpy(d.M, j.matrix, sizeof(d.M));
-    d.ray_fx = j.ray_fx; d.ray_fy = j.ray_fy; d.ray_cx = j.ray_cx; d.ray_cy = j.ray_cy;
-    d.offset_x = j.offset_x; d.offset_y = j.offset_y; d.cutoff_w2 = j.cutoff_w2;
-    d.width = j.width; d.height = j.height; d.row0 = j.row0; d.col0 = j.col0;
-    d.first_pixel = total;
-    total += (int64_t)j.width * j.height;
-  }
-  B.num_jobs = num_jobs; B.map_width = map_width; B.total_pixels = total;
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    set_error("no CUDA device: remap tables have no CPU fallback");
-    return TSCM_ERR_NO_DEVICE;
-  }
-  if (device >= 0) CUDA_TRY(cudaSetDevice(device));
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  DeviceInfo prop;
-  RC_TRY(device_info(dev, &prop));
-  if (prop.major < 10) {
-    set_error("device %d is sm_%d%d; this library is built for sm_100a only", dev, prop.major, prop.minor);
-    return TSCM_ERR_NO_DEVICE;
-  }
-  const size_t map_bytes = (size_t)map_width * map_height * sizeof(float);
-  RemapBatch* d_batch = nullptr;
-  float *d_x = nullptr, *d_y = nullptr;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  int rc = TSCM_OK;
-  auto cleanup = [&]() {
-    cudaFree(d_batch); cudaFree(d_x); cudaFree(d_y);
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-  };
-#define REMAP_TRY(expr)                                                                   \
-  do {                                                                                    \
-    cudaError_t e_ = (expr);                                                              \
-    if (e_ != cudaSuccess) {                                                              \
-      set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
-      cleanup(); return TSCM_ERR_CUDA;                                                    \
-    }                                                                                     \
-  } while (0)
-  REMAP_TRY(cudaMalloc((void**)&d_batch, sizeof(RemapBatch)));
-  REMAP_TRY(cudaMalloc((void**)&d_x, map_bytes));
-  REMAP_TRY(cudaMalloc((void**)&d_y, map_bytes));
-  REMAP_TRY(cudaMemcpy(d_batch, &B, sizeof(RemapBatch), cudaMemcpyHostToDevice));
-  REMAP_TRY(cudaEventCreate(&e0));
-  REMAP_TRY(cudaEventCreate(&e1));
-  // one wave of resident CTAs (8 x 256 threads per SM), grid-stride over the pixels
-  const int64_t want = (total + 255) / 256;
-  const int grid = (int)std::min<int64_t>(want, (int64_t)prop.sm_count * 8);
-  REMAP_TRY(cudaEventRecord(e0, 0));
-  k_remap_tables<<<grid, 256>>>(d_batch, d_x, d_y);
-  REMAP_TRY(cudaEventRecord(e1, 0));
-  REMAP_TRY(cudaGetLastError());
-  for (int k = 0; k < num_jobs && rc == TSCM_OK; ++k) {   // only the blocks that were written
-    const tscm_remap_job& j = jobs[k];
-    const size_t o = (size_t)j.row0 * map_width + j.col0, pitch = (size_t)map_width * sizeof(float);
-    REMAP_TRY(cudaMemcpy2D(mapx + o, pitch, d_x + o, pitch, (size_t)j.width * sizeof(float), j.height, cudaMemcpyDeviceToHost));
-    REMAP_TRY(cudaMemcpy2D(mapy + o, pitch, d_y + o, pitch, (size_t)j.width * sizeof(float), j.height, cudaMemcpyDeviceToHost));
-  }
-  REMAP_TRY(cudaEventSynchronize(e1));
-  if (kernel_ms) {
-    float ms = 0.f;
-    REMAP_TRY(cudaEventElapsedTime(&ms, e0, e1));
-    *kernel_ms = ms;
-  }
-#undef REMAP_TRY
-  cleanup();
-  return rc;
-}
-
-// Pose-graph initialisation (SURVEY 8f #2): multi_calib.cpp:6-153 with both candidate-scoring
-// loops on the GPU (tscm_posegraph.cuh); the O(n) pose algebra around them stays on the host.
-int tscm_pose_graph_init(const tscm_pose_graph_problem* P, int device, tscm_pose_graph_result* R) {
-  DeviceGuard device_guard_;
-  if (!P || !R || !P->worlds || !P->intrinsics || !P->has_board || !P->mono_rt || !P->pixels ||
-      !R->camera_pose || !R->board_pose || !R->board_initialised) {
-    set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT;
-  }
-  const int C = P->num_cameras, B = P->num_boards, K = P->corners_per_board;
-  if (C <= 0 || B <= 0 || K <= 0) { set_error("bad pose-graph sizes C=%d B=%d K=%d", C, B, K); return TSCM_ERR_INVALID_ARGUMENT; }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    set_error("no CUDA device: the pose-graph scoring has no CPU fallback");
-    return TSCM_ERR_NO_DEVICE;
-  }
-  if (device >= 0) CUDA_TRY(cudaSetDevice(device));
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  DeviceInfo prop;
-  RC_TRY(device_info(dev, &prop));
-  if (prop.major < 10) {
-    set_error("device %d is sm_%d%d; this library is built for sm_100a only", dev, prop.major, prop.minor);
-    return TSCM_ERR_NO_DEVICE;
-  }
-  R->kernel_ms = 0.0;
-  R->projections = 0;
-  const double nan = std::nan("");
-  if (R->camera_candidate_error) std::fill(R->camera_candidate_error, R->camera_candidate_error + (size_t)C * B, nan);
-  if (R->board_candidate_error) std::fill(R->board_candidate_error, R->board_candidate_error + (size_t)C * B, nan);
-  if (R->camera_choice) std::fill(R->camera_choice, R->camera_choice + C, -1);
-  if (R->board_choice) std::fill(R->board_choice, R->board_choice + B, -1);
-  std::fill(R->board_initialised, R->board_initialised + B, (uint8_t)0);
-
-  // device buffers, freed on every exit path
-  std::vector<void*> owned;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  auto cleanup = [&]() {
-    for (void* q : owned) cudaFree(q);
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-  };
-#define PG_TRY(expr)                                                                      \
-  do {                                                                                    \
-    cudaError_t e_ = (expr);                                                              \
-    if (e_ != cudaSuccess) {                                                              \
-      set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
-      cleanup(); return TSCM_ERR_CUDA;                                                    \
-    }                                                                                     \
-  } while (0)
-  auto dalloc = [&](void** q, size_t bytes) -> cudaError_t {
-    const cudaError_t e = cudaMalloc(q, bytes ? bytes : 8);
-    if (e == cudaSuccess) owned.push_back(*q);
-    return e;
-  };
-  const size_t px_doubles = (size_t)C * B * K * 2;
-  double *d_px = nullptr, *d_worlds = nullptr, *d_base = nullptr, *d_T = nullptr, *d_E = nullptr, *d_err = nullptr;
-  int32_t* d_shared = nullptr;
-  PG_TRY(dalloc((void**)&d_px, px_doubles * sizeof(double)));
-  PG_TRY(dalloc((void**)&d_worlds, (size_t)K * 3 * sizeof(double)));
-  PG_TRY(cudaMemcpy(d_px, P->pixels, px_doubles * sizeof(double), cudaMemcpyHostToDevice));
-  PG_TRY(cudaMemcpy(d_worlds, P->worlds, (size_t)K * 3 * sizeof(double), cudaMemcpyHostToDevice));
-  PG_TRY(dalloc((void**)&d_base, (size_t)B * 24 * sizeof(double)));
-  PG_TRY(dalloc((void**)&d_T, (size_t)B * 24 * sizeof(double)));
-  PG_TRY(dalloc((void**)&d_err, (size_t)B * sizeof(double)));
-  PG_TRY(dalloc((void**)&d_shared, (size_t)B * sizeof(int32_t)));
-  PG_TRY(cudaEventCreate(&e0));
-  PG_TRY(cudaEventCreate(&e1));
-  auto add_ms = [&]() -> cudaError_t {
-    cudaError_t e = cudaEventSynchronize(e1);
-    if (e != cudaSuccess) return e;
-    float ms = 0.f;
-    e = cudaEventElapsedTime(&ms, e0, e1);
-    R->kernel_ms += ms;
-    return e;
-  };
-
-  // ---------------- camera chain: multi_calib.cpp:14-93 ----------------
-  // candidates per pass: the (board, side) x candidate error matrix is kept below 1 GiB
-  size_t E_doubles = 0;
-  std::vector<double> cam_pose((size_t)C * 12, 0.0), base, cand, T, err;
-  std::vector<int32_t> shared;
-  for (int i = 0; i < C; ++i) {
-    double* out = cam_pose.data() + 12 * (size_t)i;
-    if (i == 0) { out[0] = out[4] = out[8] = 1.0; continue; }      // multi_calib.cpp:18-23
-    const double* camk = cam_pose.data() + 12 * (size_t)(i - 1);
-    const uint8_t *ha = P->has_board + (size_t)(i - 1) * B, *hb = P->has_board + (size_t)i * B;
-    shared.clear();
-    for (int j = 0; j < B; ++j) if (ha[j] && hb[j]) shared.push_back(j);
-    const int n = (int)shared.size();
-    if (n == 0) {
-      set_error("cameras %d and %d share no board (give the cameras in adjacent order)", i - 1, i);
-      cleanup(); return TSCM_ERR_NO_CANDIDATE;
-    }
-    base.resize((size_t)n * 24); cand.resize((size_t)n * 12); T.resize((size_t)n * 24); err.resize(n);
-    for (int f = 0; f < n; ++f) {
-      double* b = base.data() + (size_t)f * 24;
-      pg_host::split(P->mono_rt + ((size_t)i * B + shared[f]) * 9, b);             // (Ri | ti)
-      pg_host::split(P->mono_rt + ((size_t)(i - 1) * B + shared[f]) * 9, b + 12);  // (Rp | tp)
-      pg_host::chain_candidate(b, b + 12, camk, cand.data() + (size_t)f * 12);
-      pg_host::chain_transforms(camk, cand.data() + (size_t)f * 12, T.data() + (size_t)f * 24);
-    }
-    PG_TRY(cudaMemcpy(d_base, base.data(), base.size() * sizeof(double), cudaMemcpyHostToDevice));
-    PG_TRY(cudaMemcpy(d_T, T.data(), T.size() * sizeof(double), cudaMemcpyHostToDevice));
-    PG_TRY(cudaMemcpy(d_shared, shared.data(), (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice));
-    const size_t row = (size_t)2 * n;
-    int chunk = (int)std::min<size_t>((size_t)n, std::max<size_t>(kPgThreads, ((size_t)1 << 27) / row / kPgThreads * kPgThreads));
-    if (row * chunk > E_doubles) {
-      E_doubles = row * chunk;
-      PG_TRY(dalloc((void**)&d_E, E_doubles * sizeof(double)));
-    }
-    // shared boards per CTA: as many as fit 48 KB, fewer while the grid is below 8 CTAs per SM
-    int tile = 8;
-    while (tile > 1 && pg_pair_smem_bytes(K, tile) > 48 * 1024) --tile;
-    const size_t smem1 = pg_pair_smem_bytes(K, 1);
-    if (smem1 > 200 * 1024) {
-      set_error("K = %d corners per board exceed the shared-memory staging of the scoring kernel", K);
-      cleanup(); return TSCM_ERR_UNSUPPORTED;
-    }
-    if (smem1 > 48 * 1024)
-      PG_TRY(cudaFuncSetAttribute(k_pg_pair_score, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-    for (int c0 = 0; c0 < n; c0 += chunk) {
-      const int nc = std::min(chunk, n - c0);
-      const int gx = (nc + kPgThreads - 1) / kPgThreads;
-      int t = tile;
-      while (t > 1 && (int64_t)gx * ((n + t - 1) / t) < (int64_t)prop.sm_count * 8) --t;
-      if ((n + t - 1) / t > 65535) {
-        set_error("%d shared boards exceed the scoring grid (%d boards per CTA)", n, t);
-        cleanup(); return TSCM_ERR_UNSUPPORTED;
-      }
-      PgPairArgs A;
-      A.pixels = d_px; A.shared = d_shared; A.base = d_base; A.cand = d_T + (size_t)c0 * 24;
-      A.worlds = d_worlds; A.E = d_E;
-      A.intr[0] = pg_intr(P->intrinsics + 9 * (size_t)(i - 1));
-      A.intr[1] = pg_intr(P->intrinsics + 9 * (size_t)i);
-      A.cam_stride = (int64_t)B * K * 2;
-      A.cam[0] = i - 1; A.cam[1] = i;
-      A.n = n; A.nc = nc; A.K = K; A.tile = t;
-      PG_TRY(cudaEventRecord(e0, 0));
-      k_pg_pair_score<<<dim3(gx, (n + t - 1) / t), kPgThreads, pg_pair_smem_bytes(K, t)>>>(A);
-      k_pg_sum<<<gx, kPgThreads>>>(d_E, 2 * n, nc, d_err + c0);
-      PG_TRY(cudaEventRecord(e1, 0));
-      PG_TRY(cudaGetLastError());
-      PG_TRY(add_ms());
-      R->projections += (int64_t)nc * n * 2 * K;
-    }
-    PG_TRY(cudaMemcpy(err.data(), d_err, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost));
-    double min_error = 1e10;                       // multi_calib.cpp:51-52, 82-86
-    int min_id = -1;
-    for (int c = 0; c < n; ++c) {
-      if (R->camera_candidate_error) R->camera_candidate_error[(size_t)i * B + shared[c]] = err[c];
-      if (err[c] < min_error) { min_error = err[c]; min_id = c; }
-    }
-    if (min_id < 0) {
-      set_error("camera %d: none of the %d candidate poses scores below 1e10", i, n);
-      cleanup(); return TSCM_ERR_NO_CANDIDATE;
-    }
-    std::memcpy(out, cand.data() + (size_t)min_id * 12, 12 * sizeof(double));
-    if (R->camera_choice) R->camera_choice[i] = shared[min_id];
-  }
-  std::memcpy(R->camera_pose, cam_pose.data(), cam_pose.size() * sizeof(double));
-
-  // ---------------- board poses: multi_calib.cpp:95-152 ----------------
-  {
-    std::vector<double> bc((size_t)B * C * 12, 0.0), E2((size_t)B * C * C, 0.0);
-    for (int i = 0; i < B; ++i)
-      for (int j = 0; j < C; ++j) {
-        if (!P->has_board[(size_t)j * B + i]) continue;
-        double Pb[12];
-        pg_host::split(P->mono_rt + ((size_t)j * B + i) * 9, Pb);
-        pg_host::board_candidate(cam_pose.data() + 12 * (size_t)j, Pb, bc.data() + ((size_t)i * C + j) * 12);
-      }
-    double *d_bc = nullptr, *d_cam = nullptr, *d_intr = nullptr, *d_E2 = nullptr;
-    uint8_t* d_has = nullptr;
-    PG_TRY(dalloc((void**)&d_bc, bc.size() * sizeof(double)));
-    PG_TRY(dalloc((void**)&d_cam, cam_pose.size() * sizeof(double)));
-    PG_TRY(dalloc((void**)&d_intr, (size_t)C * 9 * sizeof(double)));
-    PG_TRY(dalloc((void**)&d_E2, E2.size() * sizeof(double)));
-    PG_TRY(dalloc((void**)&d_has, (size_t)C * B));
-    PG_TRY(cudaMemcpy(d_bc, bc.data(), bc.size() * sizeof(double), cudaMemcpyHostToDevice));
-    PG_TRY(cudaMemcpy(d_cam, cam_pose.data(), cam_pose.size() * sizeof(double), cudaMemcpyHostToDevice));
-    PG_TRY(cudaMemcpy(d_intr, P->intrinsics, (size_t)C * 9 * sizeof(double), cudaMemcpyHostToDevice));
-    PG_TRY(cudaMemcpy(d_has, P->has_board, (size_t)C * B, cudaMemcpyHostToDevice));
-    PG_TRY(cudaMemset(d_E2, 0, E2.size() * sizeof(double)));      // (board, candidate, camera) triples without a view stay 0
-    PgBoardArgs A;
-    A.pixels = d_px; A.has = d_has; A.cam_pose = d_cam; A.cand = d_bc; A.worlds = d_worlds; A.intr = d_intr;
-    A.E = d_E2; A.C = C; A.B = B; A.K = K;
-    const int64_t total = (int64_t)B * C * C;
-    PG_TRY(cudaEventRecord(e0, 0));
-    k_pg_board_score<<<(unsigned)((total + kPgThreads - 1) / kPgThreads), kPgThreads>>>(A);
-    PG_TRY(cudaEventRecord(e1, 0));
-    PG_TRY(cudaGetLastError());
-    PG_TRY(add_ms());
-    PG_TRY(cudaMemcpy(E2.data(), d_E2, E2.size() * sizeof(double), cudaMemcpyDeviceToHost));
-    std::vector<int> id;
-    for (int i = 0; i < B; ++i) {
-      id.clear();
-      for (int j = 0; j < C; ++j) if (P->has_board[(size_t)j * B + i]) id.push_back(j);
-      const int m = (int)id.size();
-      if (m == 0) continue;                          // multi_calib.cpp:102
-      int min_id = 0;
-      if (m > 1) {                                   // multi_calib.cpp:128-149
-        double min_error = 1e10;
-        min_id = -1;
-        for (int c = 0; c < m; ++c) {
-          double error = 0;
-          for (int k = 0; k < m; ++k) error += E2[((size_t)i * C + id[c]) * C + id[k]];
-          if (R->board_candidate_error) R->board_candidate_error[(size_t)i * C + id[c]] = error;
-          if (error < min_error) { min_error = error; min_id = c; }
-        }
-        R->projections += (int64_t)m * m * K;
-        if (min_id < 0) {
-          set_error("board %d: none of the %d candidate poses scores below 1e10", i, m);
-          cleanup(); return TSCM_ERR_NO_CANDIDATE;
-        }
-      }
-      std::memcpy(R->board_pose + 12 * (size_t)i, bc.data() + ((size_t)i * C + id[min_id]) * 12, 12 * sizeof(double));
-      R->board_initialised[i] = 1;
-      if (R->board_choice) R->board_choice[i] = id[min_id];
-    }
-  }
-#undef PG_TRY
-  cleanup();
-  return TSCM_OK;
-}
-
 int tscm_device_fp64_peak(int device, double* tflops) {
-  DeviceGuard device_guard_;
+  internal::DeviceScope device_scope;
   if (!tflops) { set_error("NULL argument"); return TSCM_ERR_INVALID_ARGUMENT; }
-  if (device >= 0) CUDA_TRY(cudaSetDevice(device));
-  DeviceInfo prop;
-  int dev = 0;
-  CUDA_TRY(cudaGetDevice(&dev));
-  RC_TRY(device_info(dev, &prop));
+  internal::SelectedDevice dev;
+  RC_TRY(internal::select_device(device, "the FP64 peak measurement", &dev));
+  internal::Scratch scratch;
   double* d_out = nullptr;
-  const int blocks = prop.sm_count * 8, threads = 256, iters = 4096;
-  CUDA_TRY(cudaMalloc((void**)&d_out, (size_t)blocks * threads * sizeof(double)));
-  cudaEvent_t e0, e1;
-  CUDA_TRY(cudaEventCreate(&e0));
-  CUDA_TRY(cudaEventCreate(&e1));
+  const int blocks = dev.sm_count * 8, threads = 256, iters = 4096;
+  CUDA_TRY(scratch.alloc(&d_out, (size_t)blocks * threads));
+  CUDA_TRY(scratch.create_events());
   double best = 0.0;
   for (int rep = 0; rep < 5; ++rep) {
-    CUDA_TRY(cudaEventRecord(e0));
+    CUDA_TRY(cudaEventRecord(scratch.e0));
     k_dfma_peak<<<blocks, threads>>>(d_out, iters, 1.0000001);
-    CUDA_TRY(cudaEventRecord(e1));
-    CUDA_TRY(cudaEventSynchronize(e1));
-    float ms = 0.f;
-    CUDA_TRY(cudaEventElapsedTime(&ms, e0, e1));
+    CUDA_TRY(cudaEventRecord(scratch.e1));
+    double ms = 0.0;
+    CUDA_TRY(scratch.add_ms(&ms));
     const double flops = 2.0 * 8.0 * (double)iters * blocks * threads;
     if (rep > 0) best = std::max(best, flops / (ms * 1e-3) / 1e12);
   }
-  cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(d_out);
   CUDA_TRY(cudaGetLastError());
   *tflops = best;
   return TSCM_OK;

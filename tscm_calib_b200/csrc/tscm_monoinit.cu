@@ -764,53 +764,24 @@ extern "C" int tscm_mono_init(const tscm_mono_init_problem* P, int device, tscm_
     internal::set_error("bad mono-init sizes: %d frames, board %d x %d (rows of at most %d corners)", F, W, H, mi::kMaxRow);
     return TSCM_ERR_INVALID_ARGUMENT;
   }
-  int sm_count = 0;
-  const int rc0 = internal::select_device(device, "the mono cold start", &sm_count);
-  if (rc0) return rc0;
+  internal::SelectedDevice dev;
+  RC_TRY(internal::select_device(device, "the mono cold start", &dev));
   R->kernel_ms = 0.0;
   R->focal_rows_used = 0;
-  std::vector<void*> owned;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  auto cleanup = [&]() {
-    for (void* q : owned) cudaFree(q);
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-  };
-#define MI_TRY(expr)                                                                      \
-  do {                                                                                    \
-    cudaError_t e_ = (expr);                                                              \
-    if (e_ != cudaSuccess) {                                                              \
-      internal::set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
-      cleanup(); return TSCM_ERR_CUDA;                                                    \
-    }                                                                                     \
-  } while (0)
-  auto dalloc = [&](void** q, size_t bytes) -> cudaError_t {
-    const cudaError_t e = cudaMalloc(q, bytes ? bytes : 8);
-    if (e == cudaSuccess) owned.push_back(*q);
-    return e;
-  };
-  auto add_ms = [&]() -> cudaError_t {
-    cudaError_t e = cudaEventSynchronize(e1);
-    if (e != cudaSuccess) return e;
-    float ms = 0.f;
-    e = cudaEventElapsedTime(&ms, e0, e1);
-    R->kernel_ms += ms;
-    return e;
-  };
+  internal::Scratch scratch;
   double *d_px = nullptr, *d_worlds = nullptr, *d_focal = nullptr, *d_rt = nullptr;
   uint8_t *d_has = nullptr, *d_ok = nullptr;
   mi::Scratch S;
   S.F = F;
-  MI_TRY(dalloc((void**)&d_px, (size_t)F * K * 2 * sizeof(double)));
-  MI_TRY(dalloc((void**)&d_worlds, (size_t)K * 3 * sizeof(double)));
-  MI_TRY(dalloc((void**)&d_has, (size_t)F));
-  MI_TRY(dalloc((void**)&d_ok, (size_t)F));
-  MI_TRY(dalloc((void**)&d_rt, (size_t)F * 9 * sizeof(double)));
-  MI_TRY(cudaMemcpy(d_px, P->pixels, (size_t)F * K * 2 * sizeof(double), cudaMemcpyHostToDevice));
-  MI_TRY(cudaMemcpy(d_worlds, P->worlds, (size_t)K * 3 * sizeof(double), cudaMemcpyHostToDevice));
-  MI_TRY(cudaMemcpy(d_has, P->has_board, (size_t)F, cudaMemcpyHostToDevice));
-  MI_TRY(cudaEventCreate(&e0));
-  MI_TRY(cudaEventCreate(&e1));
+  CUDA_TRY(scratch.alloc(&d_px, (size_t)F * K * 2));
+  CUDA_TRY(scratch.alloc(&d_worlds, (size_t)K * 3));
+  CUDA_TRY(scratch.alloc(&d_has, (size_t)F));
+  CUDA_TRY(scratch.alloc(&d_ok, (size_t)F));
+  CUDA_TRY(scratch.alloc(&d_rt, (size_t)F * 9));
+  CUDA_TRY(cudaMemcpy(d_px, P->pixels, (size_t)F * K * 2 * sizeof(double), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(d_worlds, P->worlds, (size_t)K * 3 * sizeof(double), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(d_has, P->has_board, (size_t)F, cudaMemcpyHostToDevice));
+  CUDA_TRY(scratch.create_events());
   mi::Intr I;
   if (P->has_init_guess) {                                              // TS.cpp:41
     const double* g = R->intrinsics;
@@ -818,14 +789,14 @@ extern "C" int tscm_mono_init(const tscm_mono_init_problem* P, int device, tscm_
   } else {
     // TS.cpp:43-47: integer halves of the image size, xi = lamda = 0, alpha = 0.5
     I = mi::Intr{0, 0, P->image_width / 2 - 0.5, P->image_height / 2 - 0.5, 0.0, 0.0, 0.5, 0.0, 0.0};
-    MI_TRY(dalloc((void**)&d_focal, (size_t)F * H * sizeof(double)));
-    MI_TRY(cudaEventRecord(e0, 0));
+    CUDA_TRY(scratch.alloc(&d_focal, (size_t)F * H));
+    CUDA_TRY(cudaEventRecord(scratch.e0, 0));
     mi::k_mi_focal_rows<<<(F * H + mi::kThreads - 1) / mi::kThreads, mi::kThreads>>>(d_px, d_has, F, W, H, I.cx, I.cy, d_focal);
-    MI_TRY(cudaEventRecord(e1, 0));
-    MI_TRY(cudaGetLastError());
-    MI_TRY(add_ms());
+    CUDA_TRY(cudaEventRecord(scratch.e1, 0));
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(scratch.add_ms(&R->kernel_ms));
     std::vector<double> focal((size_t)F * H);
-    MI_TRY(cudaMemcpy(focal.data(), d_focal, focal.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(focal.data(), d_focal, focal.size() * sizeof(double), cudaMemcpyDeviceToHost));
     double sum = 0;                                                     // TS.cpp:155-163, frame-major order
     int used = 0;
     for (double v : focal) if (!(v < 0)) { sum += v; ++used; }
@@ -836,28 +807,27 @@ extern "C" int tscm_mono_init(const tscm_mono_init_problem* P, int device, tscm_
   std::memcpy(R->intrinsics, out, sizeof(out));
   std::memset(R->mono_rt, 0, sizeof(double) * 9 * (size_t)F);
   std::memset(R->frame_ok, 0, (size_t)F);
-  if (!P->has_init_guess && I.fx == 0) { cleanup(); return TSCM_OK; }  // the caller returns false (TS.cpp:50)
+  if (!P->has_init_guess && I.fx == 0) return TSCM_OK;  // the caller returns false (TS.cpp:50)
   // warp-per-frame form whenever a frame's scratch fits shared memory (K <= ~350); TSCM_MI_FORM=thread
   // selects the thread-per-frame kernel, which keeps the oracle's statement order (A/B, tests)
   {
     const size_t wb = (mi::mi_warp_smem_bytes(K) + 15) & ~(size_t)15;
     const char* form = std::getenv("TSCM_MI_FORM");
     if (wb * mi::kMiWarps <= 200 * 1024 && !(form && form[0] == 't')) {
-      MI_TRY(cudaFuncSetAttribute(mi::k_mi_extrinsic_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(wb * mi::kMiWarps)));
-      MI_TRY(cudaEventRecord(e0, 0));
+      CUDA_TRY(cudaFuncSetAttribute(mi::k_mi_extrinsic_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(wb * mi::kMiWarps)));
+      CUDA_TRY(cudaEventRecord(scratch.e0, 0));
       mi::k_mi_extrinsic_warp<<<(F + mi::kMiWarps - 1) / mi::kMiWarps, 32 * mi::kMiWarps, wb * mi::kMiWarps>>>(
           d_px, d_has, d_worlds, F, W, H, I, wb, d_rt, d_ok);
-      MI_TRY(cudaEventRecord(e1, 0));
-      MI_TRY(cudaGetLastError());
-      MI_TRY(add_ms());
-      MI_TRY(cudaMemcpy(R->mono_rt, d_rt, (size_t)F * 9 * sizeof(double), cudaMemcpyDeviceToHost));
-      MI_TRY(cudaMemcpy(R->frame_ok, d_ok, (size_t)F, cudaMemcpyDeviceToHost));
-      cleanup();
+      CUDA_TRY(cudaEventRecord(scratch.e1, 0));
+      CUDA_TRY(cudaGetLastError());
+      CUDA_TRY(scratch.add_ms(&R->kernel_ms));
+      CUDA_TRY(cudaMemcpy(R->mono_rt, d_rt, (size_t)F * 9 * sizeof(double), cudaMemcpyDeviceToHost));
+      CUDA_TRY(cudaMemcpy(R->frame_ok, d_ok, (size_t)F, cudaMemcpyDeviceToHost));
       return TSCM_OK;
     }
   }
-  MI_TRY(dalloc((void**)&S.xy, (size_t)2 * K * F * sizeof(double)));
-  MI_TRY(dalloc((void**)&S.use, (size_t)K * F));
+  CUDA_TRY(scratch.alloc(&S.xy, (size_t)2 * K * F));
+  CUDA_TRY(scratch.alloc(&S.use, (size_t)K * F));
   // frames per block: as many DLT matrices as fit 200 KB of shared memory (16 at K = 88)
   const size_t a_bytes = (size_t)2 * K * 9 * sizeof(double);
   int fpb = (int)std::min<size_t>(32, (200 * 1024) / a_bytes);
@@ -866,24 +836,22 @@ extern "C" int tscm_mono_init(const tscm_mono_init_problem* P, int device, tscm_
   // an SM at `fpb` frames: it pays while all frames fit one wave (5,000 frames: 46 ms in 2.1 waves
   // against 32 ms with every frame resident at once on the global scratch).  TSCM_MI_SMEM=0/1 forces.
   const char* mode = std::getenv("TSCM_MI_SMEM");
-  const bool one_wave = fpb >= 4 && (F + fpb - 1) / fpb <= sm_count;
+  const bool one_wave = fpb >= 4 && (F + fpb - 1) / fpb <= dev.sm_count;
   S.a_in_smem = mode ? (mode[0] == '1' && fpb >= 4) : one_wave;
   size_t smem = 0;
   if (S.a_in_smem) {
     smem = a_bytes * fpb;
-    MI_TRY(cudaFuncSetAttribute(mi::k_mi_extrinsic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(cudaFuncSetAttribute(mi::k_mi_extrinsic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   } else {
     fpb = mi::kThreads;
-    MI_TRY(dalloc((void**)&S.A, a_bytes * F));
+    CUDA_TRY(scratch.alloc(&S.A, (size_t)2 * K * 9 * F));
   }
-  MI_TRY(cudaEventRecord(e0, 0));
+  CUDA_TRY(cudaEventRecord(scratch.e0, 0));
   mi::k_mi_extrinsic<<<(F + fpb - 1) / fpb, fpb, smem>>>(d_px, d_has, d_worlds, F, W, H, I, S, d_rt, d_ok);
-  MI_TRY(cudaEventRecord(e1, 0));
-  MI_TRY(cudaGetLastError());
-  MI_TRY(add_ms());
-  MI_TRY(cudaMemcpy(R->mono_rt, d_rt, (size_t)F * 9 * sizeof(double), cudaMemcpyDeviceToHost));
-  MI_TRY(cudaMemcpy(R->frame_ok, d_ok, (size_t)F, cudaMemcpyDeviceToHost));
-#undef MI_TRY
-  cleanup();
+  CUDA_TRY(cudaEventRecord(scratch.e1, 0));
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(scratch.add_ms(&R->kernel_ms));
+  CUDA_TRY(cudaMemcpy(R->mono_rt, d_rt, (size_t)F * 9 * sizeof(double), cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(R->frame_ok, d_ok, (size_t)F, cudaMemcpyDeviceToHost));
   return TSCM_OK;
 }
